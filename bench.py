@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --steps K --warmup W    (CPU arm: the reference's path on host cores)
+    python bench.py ... --dump-outputs DIR                   (also writes the last timed step's K / P / degree,
+                                                              a fixed sample of rows, as DIR/<name>.npy)
 
 One "step" = one full pass of the hot path over the synthetic Gaussian-mixture input: search operand
 -> fused distance/top-k -> float64 refine -> CSR -> symmetrise -> diffusion operator.  `value` is
@@ -43,7 +45,14 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="target CPU time of the baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write K, P and the degree vector of the last timed step to DIR/<name>.npy (GPU arm)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl %s" % a.impl)
+    return a
 
 
 def workload_name(a):
@@ -284,6 +293,45 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback"
 
 
+DUMP_ROWS = 65536          # rows of K / P written by --dump-outputs (halved until the files fit DUMP_BYTES)
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(G, out_dir, write):
+    """Writes what one build hands its caller -- kernel K (CSR), diffusion operator P (K's structure) and the degree
+    vector -- for a fixed seeded sample of rows, as float64 .npy files, so that two builds of the project can be
+    compared output for output.  rows.npy holds the sorted row ids; K_indptr / K_indices / K_data / P_data are the
+    CSR of those rows, degree.npy their row sums.  Collective when the build is row-sharded over ranks (the first
+    access of the full device matrices all-gathers them); only the rank with `write` set writes files."""
+    import torch
+    K, P, deg = G._dev_kernel, G._dev_P, G._dev_degree
+    if not write:
+        return None
+    n = K.shape[0]
+    indptr = K.indptr.cpu().numpy().astype(np.int64)
+    perm = np.random.default_rng(0).permutation(n)
+    m = min(n, DUMP_ROWS)
+    while True:
+        rows = np.sort(perm[:m])
+        lens = indptr[rows + 1] - indptr[rows]
+        nnz = int(lens.sum())
+        nbytes = 8 * (3 * nnz + 3 * m + 1) + 128 * 6           # values + one .npy header per file
+        if nbytes <= DUMP_BYTES or m == 1:
+            break
+        m //= 2
+    sub_ptr = np.concatenate([[0], np.cumsum(lens)])
+    sel = np.arange(nnz, dtype=np.int64) + np.repeat(indptr[rows] - sub_ptr[:-1], lens)
+    sel_d = torch.from_numpy(sel).to(K.data.device)
+    rows_d = torch.from_numpy(rows).to(K.data.device)
+    arrays = {"rows": rows, "K_indptr": sub_ptr, "K_indices": K.indices.index_select(0, sel_d).cpu().numpy(),
+              "K_data": K.data.index_select(0, sel_d).cpu().numpy(), "P_data": P.index_select(0, sel_d).cpu().numpy(),
+              "degree": deg.reshape(-1).index_select(0, rows_d).cpu().numpy()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
+    return {"dir": out_dir, "rows": int(m), "of": int(n), "nnz": nnz, "bytes": nbytes}
+
+
 def run_gpu_arm(a):
     import torch
     import torch.distributed as dist
@@ -367,6 +415,7 @@ def run_gpu_arm(a):
     if world > 1:
         dist.all_reduce(sums)                    # checksums / nnz of the row-sharded result, over all ranks
     checksum_K, checksum_P, nnz_sym = float(sums[0].item()), float(sums[1].item()), int(sums[2].item())
+    dumped = dump_outputs(G_last, a.dump_outputs, rank == 0) if a.dump_outputs else None
 
     # dominant kernel: fused distance/top-k; algorithmic FLOPs = 2 * Nq * Nr * d (SURVEY 8d)
     calls, search_ms = tm[SEARCH]
@@ -549,6 +598,8 @@ def run_gpu_arm(a):
             "stage_ms_source": "CUDA events around every entry point during the warm-up steps; the dominant kernel "
                                "(%s) from the events inside the timed region" % SEARCH,
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

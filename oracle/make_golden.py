@@ -16,6 +16,7 @@ from scipy import sparse
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from graphtools_b200 import synth  # noqa: E402
 from oracle.refload import load_reference  # noqa: E402
+from tests.golden_util import GOLDEN_THREADS  # noqa: E402
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
@@ -107,6 +108,8 @@ def main():
     gt = load_reference()
     assert gt is not None, "reference not available"
     import scipy, sklearn
+    from threadpoolctl import threadpool_limits
+    threadpool_limits(limits=GOLDEN_THREADS, user_api="blas")
     os.makedirs(OUT, exist_ok=True)
     for name, case in cases().items():
         if only and name not in only:
@@ -127,7 +130,7 @@ def main():
             out["sample_idx"] = np.asarray(params["sample_idx"])
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
-            G = gt.Graph(X32.astype(np.float64), n_jobs=-1, verbose=0, **params)   # keep64 inputs: already float64
+            G = gt.Graph(X32.astype(np.float64), n_jobs=GOLDEN_THREADS, verbose=0, **params)   # keep64: already f64
             if "X_from" not in case:
                 pack("K", G.kernel, out)
                 pack("P", G.diff_op, out)

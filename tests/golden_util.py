@@ -7,6 +7,12 @@ import numpy as np
 from scipy import sparse
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# Thread counts of the reference runs stored here: scikit-learn n_jobs and OpenBLAS threads, both 8.  The
+# brute-force cosine search splits the distance product over n_jobs workers and OpenBLAS splits each product over
+# its threads; either split moves the last bits of the distances, so the golden values hold for these counts and
+# not for the defaults of a host with another core count.  The runs used OpenBLAS's AVX-512 ("SkylakeX") kernels;
+# other BLAS kernels round some products differently.
+GOLDEN_THREADS = 8
 
 
 def names():

@@ -1,7 +1,7 @@
 """Host-side contract of the Data front-end (reference graphtools/base.py:72-424), mirroring the reference's own
 test/test_data.py: argument parsing, error and warning text, accepted containers, transform / inverse_transform.
-No GPU needed: graphs are created with initialize=False, and without a GPU the PCA front-end is the reference's
-scikit-learn call (GTB_PCA=auto)."""
+No GPU needed: graphs are created with initialize=False, and the PCA front-end is the reference's scikit-learn call
+(GTB_PCA=host)."""
 import numbers
 import warnings
 
@@ -14,6 +14,13 @@ from sklearn.datasets import load_digits
 import graphtools_b200 as gt
 
 DATA = load_digits().data[:400]
+
+
+@pytest.fixture(autouse=True)
+def _host_pca(monkeypatch):
+    """The host front-end on every machine: with a GPU present GTB_PCA=auto would reduce on the device, whose
+    factors agree with scikit-learn's to rounding only (tests/test_pca_gpu.py), not bit for bit."""
+    monkeypatch.setenv("GTB_PCA", "host")
 
 
 def build(data=DATA, **kw):

@@ -4,9 +4,16 @@ reproduced BIT-FOR-BIT by the oracle's restatement on the same float32-exact inp
 import numpy as np
 import pytest
 from scipy import sparse
+from threadpoolctl import threadpool_limits
 
 from oracle import graph_oracle as go
-from tests.golden_util import Case, csr_equal, names
+from tests.golden_util import GOLDEN_THREADS, Case, csr_equal, names
+
+
+@pytest.fixture(autouse=True)
+def _golden_threads():
+    with threadpool_limits(limits=GOLDEN_THREADS, user_api="blas"):
+        yield
 
 
 def _raw_kernel(case):
@@ -14,7 +21,8 @@ def _raw_kernel(case):
     if case.cls.startswith("kNN"):
         g = go.KnnOracle(X, knn=p.get("knn", 5), decay=p.get("decay", 40), knn_max=p.get("knn_max"),
                          bandwidth=p.get("bandwidth"), bandwidth_scale=p.get("bandwidth_scale", 1.0),
-                         thresh=p.get("thresh", 1e-4), distance=p.get("distance", "euclidean"))
+                         thresh=p.get("thresh", 1e-4), distance=p.get("distance", "euclidean"),
+                         n_jobs=GOLDEN_THREADS)
         return g.kernel(), g
     if case.cls.startswith("Traditional"):
         return go.exact_kernel(X, knn=p.get("knn", 5), decay=p.get("decay", 40), bandwidth=p.get("bandwidth"),
@@ -22,7 +30,7 @@ def _raw_kernel(case):
                                distance=p.get("distance", "euclidean")), None
     if case.cls.startswith("MNN"):
         return go.mnn_kernel(X, p["sample_idx"], knn=p.get("knn", 5), decay=p.get("decay", 40),
-                             thresh=p.get("thresh", 1e-4), beta=p.get("beta", 1)), None
+                             thresh=p.get("thresh", 1e-4), beta=p.get("beta", 1), n_jobs=GOLDEN_THREADS), None
     raise AssertionError(case.cls)
 
 
