@@ -78,6 +78,13 @@ _SIGS = {
     "gtb_row_scale": ([_P, _P, c_int64, c_int, c_int, _P, _P], 1),
     "gtb_slice_f64": ([_P, c_int64, c_int64, c_int64, c_int, c_int, c_int64, c_int64, _P, _P, _P], 2),
     "gtb_gemm_i8": ([_P, _P, c_int, c_int64, c_int64, c_int64, c_int64, c_int64, _P, _P, _P, c_int64, c_int, _P], 1),
+    "gtb_dense_to_csr_count": ([_P, c_int64, c_int64, _P, _P], 1),
+    "gtb_dense_to_csr_fill": ([_P, c_int64, c_int64, _P, _P, _P, _P], 1),
+    "gtb_sp_lengths": ([_P, _P, _P, c_int64, _P, c_int, c_int, c_int, _P, _P, _P], 1),
+    "gtb_sp_components": ([_P, _P, c_int64, _P, _P], 3),
+    "gtb_sp_traverse": ([_P, _P, _P, c_int64, _P, c_int, c_int, _P, _P, _P], 1),
+    "gtb_sp_store_rows": ([_P, c_int, c_int64, _P, c_int, _P, c_int64, _P], 1),
+    "gtb_sp_finish": ([_P, c_int64, _P], 1),
 }
 _PLAIN = {
     "gtb_last_error": ([], ctypes.c_char_p),
@@ -91,6 +98,7 @@ _PLAIN = {
     "gtb_tc_scratch_bytes": ([c_int64], c_int64),
     "gtb_gemm_max_k": ([], c_int),
     "gtb_knn_seed_k": ([], c_int),
+    "gtb_sp_ws_bytes": ([c_int64, c_int], c_int64),
 }
 
 

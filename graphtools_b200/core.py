@@ -576,6 +576,25 @@ class BaseGraph(Base, metaclass=abc.ABCMeta):
         x = x.cpu().numpy()
         return x[:, 0] if one_d else x
 
+    @property
+    def weighted(self):
+        """True when the kernel holds affinities (``decay is not None``) rather than a binary adjacency."""
+        return getattr(self, "decay", None) is not None
+
+    def shortest_path(self, method="auto", distance=None):
+        """Length of the shortest path between every pair of vertices (reference base.py:934-988), float64 [N, N].
+
+        ``distance`` sets the edge lengths on every stored entry of K: "constant" (K_ij itself; unweighted graphs),
+        "data" (Euclidean distance between the rows of ``data_nu``; unweighted graphs) or "affinity" (-log K_ij;
+        weighted graphs); None picks "data" for unweighted and "affinity" for weighted graphs.  Paths are directed
+        along K's rows; the result is then averaged with its transpose, pairs at distance 0 (duplicate points) or
+        without a path get inf, and the diagonal is 0.  ``method`` is checked against scipy's names ("auto", "FW",
+        "D", "BF", "J"); every method yields the float64 fixpoint of the edge relaxations, which is bit-identical
+        to scipy's Dijkstra (FW rounds differently, within 1e-12 relative).  Negative lengths (affinities above 1,
+        possible with anisotropy > 0) raise NotImplementedError.  Runs on the device (csrc/paths.cu)."""
+        from . import paths
+        return paths.shortest_path(self, method=method, distance=distance)
+
     @staticmethod
     def _materialize(dev):
         if isinstance(dev, pipeline.DeviceCSR):

@@ -13,4 +13,4 @@ void gtb_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* gtb_last_error(void) { return g_err; }
-extern "C" int gtb_version(void) { return 200; }   // round-2 ABI (seeded search, split operand preparation, int8 GEMM)
+extern "C" int gtb_version(void) { return 201; }   // + K10 all-pairs shortest paths (gtb_sp_*, gtb_dense_to_csr_*)

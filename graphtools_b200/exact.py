@@ -74,6 +74,16 @@ class TraditionalGraph(DataGraph):
         super().set_params(**params)
         return self
 
+    @property
+    def weighted(self):
+        """Precomputed graphs: True when K has a non-zero value outside {0.5, 1} (a symmetrised binary adjacency
+        holds only those); graphs built from data: ``decay is not None``."""
+        if self.precomputed is None:
+            return super().weighted
+        K = self.K
+        vals = K.data if sparse.issparse(K) else K[K != 0]
+        return not bool(np.all(np.isin(vals, [0.5, 1.0])))
+
     # ------------------------------------------------------------------ device side
     def _metric(self):
         return self.distance if self.precomputed is None else "euclidean"

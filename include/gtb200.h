@@ -285,6 +285,32 @@ int gtb_gemm_i8(const int8_t* a_digits, const int8_t* b_digits, int slices, int6
                 int64_t M_pad, int64_t N_pad, const double* sa, const double* sb, double* C, int64_t ldc,
                 int row_bytes, void* stream);
 
+/* ---- K10 all-pairs shortest paths: replaces scipy.sparse.csgraph.shortest_path behind BaseGraph.shortest_path
+ * (base.py:934-988) ---------------------------------------------------------------------------------------------- */
+/* Present (non-zero) entries of a dense float64 matrix as a column-sorted CSR, what csr_matrix(K) stores:
+ * count -> gtb_exclusive_scan -> fill */
+int gtb_dense_to_csr_count(const double* K, int64_t n_rows, int64_t n_cols, int32_t* cnt, void* stream);
+int gtb_dense_to_csr_fill(const double* K, int64_t n_rows, int64_t n_cols, const int64_t* indptr, int32_t* idx,
+                          double* val, void* stream);
+/* len[nnz] = edge length of every stored entry: mode 0 K_ij, 1 |x_i - x_j|_2 of the rows X[n][d] (float32, or float64
+ * when x_is_f64; numpy's pairwise summation order in that dtype), 2 -log(K_ij) correctly rounded.  *flags |= 1 when a
+ * length is negative or NaN (the caller zeroes flags) */
+int gtb_sp_lengths(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const void* X, int d,
+                   int x_is_f64, int mode, double* len, int32_t* flags, void* stream);
+/* label[n] = smallest vertex of the weakly connected component (union-find over the stored entries) */
+int gtb_sp_components(const int64_t* indptr, const int32_t* idx, int64_t n, int32_t* label, void* stream);
+/* dist[n][batch] = shortest-path lengths from the nb <= batch sources src[] (column b: source src[b], +inf where
+ * unreachable); batch is a multiple of 32, at most 1024; ws: gtb_sp_ws_bytes(n, batch) bytes.  Lengths must be
+ * non-negative.  One cooperative launch (grid-wide barriers between relaxation rounds). */
+int64_t gtb_sp_ws_bytes(int64_t n, int batch);
+int gtb_sp_traverse(const int64_t* indptr, const int32_t* idx, const double* len, int64_t n, const int32_t* src, int nb,
+                    int batch, double* dist, void* ws, void* stream);
+/* out[src[b]][v] = dist[v][b] for b < nb (row stride ldo) */
+int gtb_sp_store_rows(const double* dist, int batch, int64_t n, const int32_t* src, int nb, double* out, int64_t ldo,
+                      void* stream);
+/* in place on D[n][n]: (D + D^T) / 2, then 0 -> +inf off the diagonal, 0 on the diagonal */
+int gtb_sp_finish(double* D, int64_t n, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
