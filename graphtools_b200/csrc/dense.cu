@@ -98,7 +98,8 @@ __global__ void __launch_bounds__(256) dense_kernel(const T* __restrict__ Xq, in
         if (j >= nr) continue;
         double dist;
         if (metric == 1) {
-          double c = acc[a][b] / (sqrt(qn[a]) * sqrt(rn[b]));
+          // an all-zero row has no direction: NaN, as in scipy (the kernel below maps it to 1 like the reference)
+          double c = (qn[a] == 0.0 || rn[b] == 0.0) ? NAN : acc[a][b] / (sqrt(qn[a]) * sqrt(rn[b]));
           if (fabs(c) > 1.0) c = copysign(1.0, c);
           dist = 1.0 - c;
         } else if (metric == 2) {
@@ -111,16 +112,17 @@ __global__ void __launch_bounds__(256) dense_kernel(const T* __restrict__ Xq, in
           v = dist;
         } else {
           // pairs beyond the kernel support radius bw * (-ln thresh)^(1/decay) are zero: skip pow/exp
-          // (the 1e-9 guard keeps every value that could round to >= thresh on the exact path)
+          // (the 1e-9 guard keeps every value that could round to >= thresh on the exact path); a NaN distance or
+          // bandwidth passes the test and gtb_affinity turns it into 1, np.where(isnan(K), 1, K) in the reference
           v = 0.0;
-          if (dist <= bwi * rfac) {
+          if (!(dist > bwi * rfac)) {
             v = gtb_affinity(dist, bwi, decay);
             if (v < thresh) v = 0.0;
           }
           if (what == DENSE_KERNEL_SYM) {
             double vr = 0.0;
             const double bwj = bw_r[j];
-            if (dist <= bwj * rfac) {
+            if (!(dist > bwj * rfac)) {
               vr = gtb_affinity(dist, bwj, decay);
               if (vr < thresh) vr = 0.0;
             }

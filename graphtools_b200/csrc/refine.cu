@@ -73,7 +73,8 @@ __device__ __forceinline__ double search2_of_radius(double r, int metric) {
   return metric == 0 ? r * r : (metric == 1 ? 2.0 * r : r);
 }
 
-// squared cosine distance between two rows of the ORIGINAL data, float64, one warp
+// squared cosine distance between two rows of the ORIGINAL data, float64, one warp.  An all-zero row is at
+// distance 1 from every row, itself included: sklearn's normalize leaves it at zero, so its dot products are 0.
 template <typename T>
 __device__ __forceinline__ double warp_cos2(const T* __restrict__ xq, const T* __restrict__ xr, int d, int lane) {
   double dot = 0.0, nx = 0.0, ny = 0.0;
@@ -87,6 +88,7 @@ __device__ __forceinline__ double warp_cos2(const T* __restrict__ xq, const T* _
     nx += __shfl_xor_sync(0xffffffffu, nx, off);
     ny += __shfl_xor_sync(0xffffffffu, ny, off);
   }
+  if (nx == 0.0 || ny == 0.0) return 1.0;
   double dc = 1.0 - dot / (sqrt(nx) * sqrt(ny));
   dc = fmin(fmax(dc, 0.0), 2.0);          // np.clip(S, 0, 2) in sklearn cosine_distances
   return dc * dc;

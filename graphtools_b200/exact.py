@@ -95,12 +95,35 @@ class TraditionalGraph(DataGraph):
             self._dev_X = self._dense_f32(self.data_nu)
         return self._dev_X
 
+    def _zero_rows(self, X):
+        """Rows of ``X`` that are all zero, for the cosine metric (None otherwise): scipy's cosine distance from such
+        a row is NaN."""
+        if self._metric() != "cosine":
+            return None
+        return (X == 0).all(dim=1)
+
     def _adaptive_bandwidth(self, Xq_op, ref_op, knn_eff):
         """Distance to the knn_eff-th nearest reference point (self counted when in-sample):
-        np.partition(pdx, k)[:, :k].max (graphs.py:1583-1587, :1655-1656)."""
-        _, info = pipeline.knn_kernel(None, ref_op, Xq_op, knn=knn_eff, decay=max(float(self.decay), 1.0),
-                                      thresh=0.5, bandwidth_scale=1.0)
-        return info["bandwidth"]
+        np.partition(pdx, k)[:, :k].max (graphs.py:1583-1587, :1655-1656).
+
+        Cosine with all-zero rows: their distances are NaN in the reference, which np.partition sorts last. So the
+        neighbours are searched among the non-zero reference rows, and the bandwidth is NaN where the k smallest
+        entries of a row include a NaN: every zero query row, and every row when fewer than k reference rows are
+        non-zero."""
+        zq, zr = self._zero_rows(Xq_op.X), self._zero_rows(ref_op.X)
+        if zq is None or not bool(zq.any().item() or zr.any().item()):
+            _, info = pipeline.knn_kernel(None, ref_op, Xq_op, knn=knn_eff, decay=max(float(self.decay), 1.0),
+                                          thresh=0.5, bandwidth_scale=1.0)
+            return info["bandwidth"]
+        bw = torch.full((Xq_op.n,), float("nan"), dtype=torch.float64, device=Xq_op.X.device)
+        keep_r, keep_q = (~zr).nonzero().flatten(), (~zq).nonzero().flatten()
+        if keep_r.shape[0] >= knn_eff and keep_q.shape[0] > 0:
+            ref_nz = pipeline.SearchOperand(ref_op.X[keep_r].contiguous(), metric="cosine")
+            qry_nz = pipeline.SearchOperand(Xq_op.X[keep_q].contiguous(), mean=ref_nz.mean, metric="cosine")
+            _, info = pipeline.knn_kernel(None, ref_nz, qry_nz, knn=knn_eff, decay=max(float(self.decay), 1.0),
+                                          thresh=0.5, bandwidth_scale=1.0)
+            bw[keep_q] = info["bandwidth"]
+        return bw
 
     def _resolve_bandwidth(self, bandwidth, n_rows, dist_fn, Xq_op, ref_op, knn_eff):
         dev = pipeline._dev()
@@ -138,8 +161,12 @@ class TraditionalGraph(DataGraph):
         """With a positive threshold the exact kernel has the same support as the kNN-graph kernel without
         knn_max (all j with exp(-(d/bw)^decay) >= thresh), so it is built sparse on the tensor-core
         search path and densified once; thresh == 0 or a callable bandwidth need every pair -> dense kernel."""
-        return (self.thresh is not None and self.thresh > 0 and self.decay is not None
-                and not callable(self.bandwidth) and self.knn is not None and self.knn + 1 + 8 <= 128)
+        if not (self.thresh is not None and self.thresh > 0 and self.decay is not None
+                and not callable(self.bandwidth) and self.knn is not None and self.knn + 1 + 8 <= 128):
+            return False
+        # a zero row under the cosine metric has NaN distances, i.e. affinity 1 to every sample: not sparse
+        zero = self._zero_rows(self._X())
+        return zero is None or not bool(zero.any().item())
 
     def _build_kernel_via_sparse(self):
         from . import _engine as E

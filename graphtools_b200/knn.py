@@ -14,6 +14,63 @@ from .core import DataGraph
 from .logging_util import logger as _logger
 
 
+def search_schedule(count_ge, nq, n_ref, knn, knn_max, search_multiplier):
+    """Replay of the reference's search escalation (graphs.py:882-948) from neighbour counts.
+
+    ``count_ge(s)`` is the number of query rows (all ``nq`` of them, over every rank) with at least ``s`` reference
+    points strictly inside their kernel radius.  The reference searches ``s`` neighbours per row and keeps a row to do
+    when all ``s`` lie inside the radius, i.e. exactly when its count is >= s; whether it searches wider follows from
+    the number of such rows.  Returns ``(s_todo, search_knn, n_todo)``: after the last kNN pass the rows with a count
+    >= ``s_todo`` are still to do (``n_todo`` of them), and ``search_knn`` is the width of the step that finishes
+    them.  When ``search_knn > n_ref / 2`` the reference finishes those rows on a new brute-force search built without
+    its ``metric`` argument, i.e. with Euclidean distances."""
+    knn = min(knn, n_ref)
+    knn_max = n_ref if knn_max is None else knn_max
+    s = min(knn * search_multiplier, knn_max)
+    s_todo, n_todo = s, count_ge(s)
+    s_next = min(s * search_multiplier, knn_max)
+    while n_todo > nq // 10 and s_next < n_ref / 2 and s_next < knn_max and s_next > s_todo:
+        s_todo, n_todo = s_next, count_ge(s_next)
+        s_next = min(s_next * search_multiplier, knn_max)
+    return s_todo, s_next, n_todo
+
+
+def _schedule_widths(n_ref, knn, knn_max, search_multiplier):
+    """Every search width ``search_schedule`` can ask ``count_ge`` about, in order."""
+    knn = min(knn, n_ref)
+    knn_max = n_ref if knn_max is None else knn_max
+    s = min(knn * search_multiplier, knn_max)
+    widths = [s]
+    s = min(s * search_multiplier, knn_max)
+    while s < n_ref / 2 and s < knn_max and s > widths[-1]:
+        widths.append(s)
+        s = min(s * search_multiplier, knn_max)
+    return widths
+
+
+def _splice_rows(R, rows, R2):
+    """DeviceCSR ``R`` with its rows ``rows`` (int64 device tensor) replaced by the rows of ``R2``, in that order.
+    Rows of both matrices are sorted by column, so a stable sort of all entries by row keeps them sorted."""
+    import torch
+    n = R.shape[0]
+    dev = R.indices.device
+    lens = R.indptr[1:] - R.indptr[:-1]
+    lens2 = R2.indptr[1:] - R2.indptr[:-1]
+    replaced = torch.zeros((n,), dtype=torch.bool, device=dev)
+    replaced[rows] = True
+    row_of = torch.repeat_interleave(torch.arange(n, device=dev), lens)
+    keep = ~replaced[row_of]
+    all_rows = torch.cat([row_of[keep], torch.repeat_interleave(rows, lens2)])
+    order = torch.argsort(all_rows, stable=True)
+    idx = torch.cat([R.indices[keep], R2.indices])[order].contiguous()
+    val = torch.cat([R.data[keep], R2.data])[order].contiguous()
+    new_lens = lens.clone()
+    new_lens[rows] = lens2
+    indptr = torch.zeros((n + 1,), dtype=torch.int64, device=dev)
+    torch.cumsum(new_lens, dim=0, out=indptr[1:])
+    return pipeline.DeviceCSR(indptr, idx, val, R.shape)
+
+
 class kNNGraph(DataGraph):
     """K nearest neighbours graph, optionally with alpha-decay affinities."""
 
@@ -143,10 +200,12 @@ class kNNGraph(DataGraph):
         if hi > lo:
             qry = pipeline.SearchOperand(Xq[lo:hi], mean=ref.mean, metric=ref.metric)
             Rl, info = self._kernel_device(qry, ref, knn=knn, knn_max=knn_max, bandwidth=bandwidth,
-                                           bandwidth_scale=bandwidth_scale)
+                                           bandwidth_scale=bandwidth_scale, nq_total=Xq.shape[0])
             return (bounds, Rl.indptr, (Rl.indptr[1:] - Rl.indptr[:-1]).to(torch.int32), Rl.indices, Rl.data,
                     info)
         z = torch.zeros((0,), dtype=torch.int32, device=dev)
+        if ref.metric != "euclidean" and not (self.decay is None or self.thresh == 1):
+            self._fallback_plan(z, ref.n, knn, knn_max, Xq.shape[0])      # the other ranks' replay is collective
         return (bounds, torch.zeros((1,), dtype=torch.int64, device=dev), z, z,
                 torch.zeros((0,), dtype=torch.float64, device=dev), {"nzero": z, "bandwidth": None})
 
@@ -211,11 +270,57 @@ class kNNGraph(DataGraph):
         pipeline._STATS.update(nnz_sym_local=int(k_idx.shape[0]))
         return None
 
-    def _kernel_device(self, qry, ref, knn, knn_max, bandwidth, bandwidth_scale):
+    def _kernel_device(self, qry, ref, knn, knn_max, bandwidth, bandwidth_scale, nq_total=None):
+        """Raw kernel rows of ``qry`` against ``ref``.  ``nq_total``: the query rows are this rank's shard of that
+        many rows (the search schedule is then replayed on counts summed over the ranks)."""
         if self.decay is None or self.thresh == 1:
             return pipeline.knn_kernel(None, ref, qry, knn=knn, knn_max=None, decay=None)
-        return pipeline.knn_kernel(None, ref, qry, knn=knn, knn_max=knn_max, decay=self.decay,
-                                   thresh=self.thresh, bandwidth=bandwidth, bandwidth_scale=bandwidth_scale)
+        R, info = pipeline.knn_kernel(None, ref, qry, knn=knn, knn_max=knn_max, decay=self.decay,
+                                      thresh=self.thresh, bandwidth=bandwidth, bandwidth_scale=bandwidth_scale)
+        if ref.metric != "euclidean":
+            R = self._euclidean_fallback(R, info, qry, ref, knn, knn_max, nq_total)
+        return R, info
+
+    def _fallback_plan(self, row_len, n_ref, knn, knn_max, nq_total):
+        """(s_todo, search_knn, n_todo) of ``search_schedule`` from the raw row lengths of this rank's query rows
+        (the number of reference points inside each row's radius, capped at knn_max); the counts are summed over
+        the ranks when ``nq_total`` is given.  Collective in that case: every rank calls it, also with no rows."""
+        import torch
+        widths = _schedule_widths(n_ref, knn, knn_max, self.search_multiplier)
+        ge = torch.stack([(row_len >= s).sum() for s in widths]).to(torch.int64)
+        if nq_total is not None:
+            import torch.distributed as dist
+            dist.all_reduce(ge)
+        at = dict(zip(widths, ge.tolist()))
+        nq = row_len.shape[0] if nq_total is None else nq_total
+        return search_schedule(at.__getitem__, nq, n_ref, knn, knn_max, self.search_multiplier)
+
+    def _euclidean_fallback(self, R, info, qry, ref, knn, knn_max, nq_total=None):
+        """Reference quirk H9 (graphs.py:945-948): when its search escalates beyond N/2 neighbours, the rows still
+        to do are searched on a brute-force index built WITHOUT ``metric=``.  Their kernel rows then hold Euclidean
+        distances divided by the metric's own bandwidth: the radius search, or the ``knn_max`` nearest when the
+        search width has reached knn_max.  The schedule is replayed from the metric rows' lengths and those rows
+        are rebuilt on a Euclidean operand of the same data."""
+        row_len = R.indptr[1:] - R.indptr[:-1]
+        s_todo, s_final, n_todo = self._fallback_plan(row_len, ref.n, knn, knn_max, nq_total)
+        if not (s_final > ref.n / 2 and n_todo > 0):
+            return R
+        rows = (row_len >= s_todo).nonzero().flatten()
+        main_stats = dict(pipeline._STATS, euclidean_fallback_rows=int(n_todo))
+        if rows.shape[0] == 0:
+            pipeline._STATS.update(main_stats)
+            return R
+        if getattr(self, "_euclid_ref", None) is None or self._euclid_ref[0] is not ref:
+            self._euclid_ref = (ref, pipeline.SearchOperand(ref.X, metric="euclidean"))
+        eref = self._euclid_ref[1]
+        sub = pipeline.SearchOperand(qry.X[rows].contiguous(), mean=eref.mean, metric="euclidean")
+        bw = info["bandwidth"][rows].cpu().numpy()
+        kmax = ref.n if knn_max is None else knn_max
+        R2, _ = pipeline.knn_kernel(None, eref, sub, knn=knn, knn_max=kmax if s_final == kmax else None,
+                                    decay=self.decay, thresh=self.thresh, bandwidth=bw, bandwidth_scale=1.0)
+        pipeline._STATS.clear()
+        pipeline._STATS.update(main_stats)           # stats() describes the metric search, plus the rebuilt rows
+        return _splice_rows(R, rows, R2)
 
     def _check_duplicates(self, info, qry, ref):
         """Warn about zero distances between distinct samples (graphs.py:787-817)."""

@@ -159,7 +159,9 @@ class SearchOperand:
 
         metric="cosine": the search copy is built from the row-normalised data (normalised and centred in float64,
         rounded once), on which squared Euclidean distance = 2 x cosine distance; the exact stage evaluates
-        1 - x.y / (|x||y|) on the original rows."""
+        1 - x.y / (|x||y|) on the original rows.  All-zero rows stay zero, as in sklearn's ``normalize``; their
+        search distance to a normalised row is 1 (to another zero row 0), below the 2 x 1 of their exact cosine
+        distance, so the certification bounds stay conservative for them."""
         n, d = X.shape
         self.X, self.n, self.d = X, n, d
         self.metric = metric
@@ -180,7 +182,8 @@ class SearchOperand:
         elif self.is64 or metric == "cosine":
             rows = X.to(torch.float64)
             if metric == "cosine":
-                rows = rows / rows.norm(dim=1, keepdim=True)
+                norms = rows.norm(dim=1, keepdim=True)
+                rows = rows / torch.where(norms > 0, norms, torch.ones_like(norms))
             if mean is None:
                 mean = rows.mean(dim=0)
             self.Xs = (rows - mean.to(torch.float64)).to(torch.float32).contiguous()
@@ -604,7 +607,7 @@ def knn_kernel(Xq, ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, b
     count = _empty((1,), torch.int32)
     E.call("gtb_compact_todo", status, nq, todo_rows, count)
     nt = int(count.item())                       # host sync #1
-    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=impl)
+    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=impl, euclidean_fallback_rows=0)
 
     seg_ptr = seg_idx = seg_val = n_keep_t = None
     if nt > 0:

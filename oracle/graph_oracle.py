@@ -98,6 +98,10 @@ class KnnOracle:
         self.distance, self.thresh, self.n_jobs = distance, thresh, n_jobs
         self._tree = None
         self.passes = []  # (search_knn, rows searched) per kNN pass, for reporting
+        # per kernel_to_data call with a decay: dict(todo=rows still to do after the last kNN pass,
+        # search_knn=width of the final step, fallback=that step ran on the metric-less brute-force index,
+        # branch="kneighbors" | "radius" | None)
+        self.schedules = []
 
     @property
     def tree(self):                                         # graphs.py:748-769
@@ -150,6 +154,9 @@ class KnnOracle:
             far = np.fromiter((r.max() for r in dist), dtype=np.float64, count=len(dist))
             todo = np.flatnonzero(far < radius)
             search_knn = min(search_knn * mult, knn_max)
+        self.schedules.append(dict(todo=todo.copy(), search_knn=search_knn, fallback=search_knn > n_ref / 2,
+                                   branch=(None if todo.size == 0 else
+                                           "kneighbors" if search_knn == knn_max else "radius")))
         if search_knn > n_ref / 2:                          # graphs.py:945-948 (no metric!)
             tree = NearestNeighbors(n_neighbors=search_knn, algorithm="brute",
                                     n_jobs=self.n_jobs).fit(self.data)

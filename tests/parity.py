@@ -20,12 +20,14 @@ def _coo_keys(M):
 def _tie_exempt(rows, cols, X, knn_eff, Y=None, metric="euclidean"):
     """True where entry (i, j) sits on a k-th / (k+1)-th neighbour tie (north_star: distances within
     1e-6 relative) in row i -- or in row j for symmetrised in-sample graphs (Y is None).  Cosine ties are
-    ties of the Euclidean distance between the normalised rows (d_euc^2 = 2 d_cos)."""
+    ties of the Euclidean distance between the rows normalised as sklearn's ``normalize`` does (d_euc^2 = 2 d_cos;
+    all-zero rows stay zero)."""
+    from sklearn.preprocessing import normalize
     X = np.asarray(X, dtype=np.float64)
     Q = X if Y is None else np.asarray(Y, dtype=np.float64)
     if metric == "cosine":
-        Xn = X / np.linalg.norm(X, axis=1, keepdims=True)
-        Q = Xn if Y is None else Q / np.linalg.norm(Q, axis=1, keepdims=True)
+        Xn = normalize(X)
+        Q = Xn if Y is None else normalize(Q)
         X = Xn
     ok = np.zeros(len(rows), dtype=bool)
     cache = {}
