@@ -13,4 +13,4 @@ void gtb_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* gtb_last_error(void) { return g_err; }
-extern "C" int gtb_version(void) { return 201; }   // + K10 all-pairs shortest paths (gtb_sp_*, gtb_dense_to_csr_*)
+extern "C" int gtb_version(void) { return 202; }   // + sqeuclidean and correlation metrics (x_kind bits 1-3, dense metric 3)

@@ -7,7 +7,8 @@
 // branches of symmetrize_kernel / apply_anisotropy / normalize (base.py:557-592, :645).
 // Distances are float64 direct differences of the inputs as given -- float32 rows or float64 rows (PCA output,
 // float64 user data), template T -- which is what scipy's pdist / cdist compute.  Metrics: euclidean, cosine,
-// cityblock.  Row sums are NOT accumulated here (a floating-point atomic per tile would make the degree vector
+// cityblock, sqeuclidean (correlation is the cosine branch on row-centred float64 rows, prepared by the caller as
+// scipy does).  Row sums are NOT accumulated here (a floating-point atomic per tile would make the degree vector
 // depend on the tile order): gtb_dense_rowsum makes one deterministic pass afterwards.
 #include "common.cuh"
 #include "gtb200.h"
@@ -102,7 +103,7 @@ __global__ void __launch_bounds__(256) dense_kernel(const T* __restrict__ Xq, in
           double c = (qn[a] == 0.0 || rn[b] == 0.0) ? NAN : acc[a][b] / (sqrt(qn[a]) * sqrt(rn[b]));
           if (fabs(c) > 1.0) c = copysign(1.0, c);
           dist = 1.0 - c;
-        } else if (metric == 2) {
+        } else if (metric == 2 || metric == 3) {
           dist = acc[a][b];
         } else {
           dist = sqrt(acc[a][b]);
@@ -183,7 +184,7 @@ extern "C" int gtb_dense_kernel(const void* Xq, int64_t nq, const void* Xr, int6
                                 double theta, double* out, double* rowsum, void* stream) {
   GTB_CHECK_ARG(nq > 0 && nr > 0 && d > 0, "empty input");
   GTB_CHECK_ARG(what >= 0 && what <= 2, "bad mode");
-  GTB_CHECK_ARG(metric >= 0 && metric <= 2, "metric must be 0 (euclidean), 1 (cosine) or 2 (cityblock)");
+  GTB_CHECK_ARG(metric >= 0 && metric <= 3, "metric must be 0 (euclidean), 1 (cosine), 2 (cityblock) or 3 (sqeuclidean)");
   GTB_CHECK_ARG(what == 0 || bw_q != nullptr, "bandwidth required");
   GTB_CHECK_ARG(what != 2 || (bw_r != nullptr && nq == nr), "symmetric mode needs a square problem");
   cudaStream_t st = (cudaStream_t)stream;

@@ -26,8 +26,12 @@ struct RowParams {
   const double* bw_fixed; int bw_mode;  // 0 adaptive (k-th neighbour), 1 scalar, 2 per-row
   double bw_scale; double bw_floor;     // bw_floor = eps (np.finfo(float).eps)
   int metric;                           // 0 euclidean, 1 cosine (1 - x.y / (|x||y|), sklearn cosine_distances),
-                                        // 2 cityblock (sum |x - y|, sklearn manhattan_distances)
+                                        // 2 cityblock (sum |x - y|, sklearn manhattan_distances),
+                                        // 3 sqeuclidean (sum (x - y)^2), 4 correlation (cosine of the row-centred rows)
 };
+
+// metrics whose exact stage evaluates the Euclidean sum s = sum (x - y)^2 on the fast gather paths below
+__host__ __device__ __forceinline__ bool euclidean_sum(int metric) { return metric == 0 || metric == 3; }
 
 // exact squared distance between query row xq and reference row xr, cooperatively by one warp
 // (float32 rows made of whole, 16-byte aligned float4s are read as float4 -- the same element-to-lane assignment and
@@ -66,11 +70,14 @@ __device__ __forceinline__ double warp_dist2(const T* __restrict__ xq, const T* 
 // ordering, and the certification arithmetic below converts between the metric's own units (in which key[] holds the
 // SQUARED exact distance, so sqrt(key) is the distance for both metrics) and search-space squared distances.
 // Cityblock: the fast pass accumulates sum |x - y| itself, so the search-space value IS the distance.
+// Correlation: cosine of the row-centred rows, searched like cosine on the centred, row-normalised copies.
+// Sqeuclidean: the fast pass is the Euclidean one and key = s^2 for the Euclidean sum s (the distance), so
+// sqrt(key) == s exactly (binary64, no overflow or underflow) is both the distance and its search-space value.
 __device__ __forceinline__ double search2_of_key(double key, int metric) {
-  return metric == 0 ? key : (metric == 1 ? 2.0 * sqrt(key) : sqrt(key));
+  return metric == 0 ? key : ((metric == 1 || metric == 4) ? 2.0 * sqrt(key) : sqrt(key));
 }
 __device__ __forceinline__ double search2_of_radius(double r, int metric) {
-  return metric == 0 ? r * r : (metric == 1 ? 2.0 * r : r);
+  return metric == 0 ? r * r : ((metric == 1 || metric == 4) ? 2.0 * r : r);
 }
 
 // squared cosine distance between two rows of the ORIGINAL data, float64, one warp.  An all-zero row is at
@@ -94,6 +101,42 @@ __device__ __forceinline__ double warp_cos2(const T* __restrict__ xq, const T* _
   return dc * dc;
 }
 
+// float64 mean of one row of the ORIGINAL data, one warp (scipy's correlation centres each row by its np.mean)
+template <typename T>
+__device__ __forceinline__ double warp_mean(const T* __restrict__ x, int d, int lane) {
+  double s = 0.0;
+  for (int k = lane; k < d; k += 32) s += (double)x[k];
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+  return s / d;
+}
+
+// squared correlation distance between query row xq (row mean mq) and reference row xr of the ORIGINAL data, float64,
+// one warp: the mean of xr first, then the centred dot product and norms on a second pass over the row (now in L1).
+// A constant row (centred row zero) is rejected by the host before any search; like an all-zero cosine row it would
+// be at distance 1 from every row.  Not inlined: inlined, it raises refine_ball_kernel<float> from 48 to 58 registers
+// for every metric, the Euclidean one included.
+template <typename T>
+__device__ __noinline__ double warp_corr2(const T* __restrict__ xq, double mq, const T* __restrict__ xr, int d,
+                                             int lane) {
+  const double mr = warp_mean<T>(xr, d, lane);
+  double dot = 0.0, nx = 0.0, ny = 0.0;
+  for (int k = lane; k < d; k += 32) {
+    const double a = (double)xq[k] - mq, b = (double)xr[k] - mr;
+    dot = fma(a, b, dot); nx = fma(a, a, nx); ny = fma(b, b, ny);
+  }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) {
+    dot += __shfl_xor_sync(0xffffffffu, dot, off);
+    nx += __shfl_xor_sync(0xffffffffu, nx, off);
+    ny += __shfl_xor_sync(0xffffffffu, ny, off);
+  }
+  if (nx == 0.0 || ny == 0.0) return 1.0;
+  double dc = 1.0 - dot / (sqrt(nx) * sqrt(ny));
+  dc = fmin(fmax(dc, 0.0), 2.0);
+  return dc * dc;
+}
+
 // squared cityblock distance between two rows of the ORIGINAL data, float64, one warp
 template <typename T>
 __device__ __forceinline__ double warp_l1sq(const T* __restrict__ xq, const T* __restrict__ xr, int d, int lane) {
@@ -104,8 +147,10 @@ __device__ __forceinline__ double warp_l1sq(const T* __restrict__ xq, const T* _
   return s * s;
 }
 
+// cosine, cityblock, correlation (mq: the query row's mean, read by correlation only)
 template <typename T>
-__device__ __forceinline__ double warp_metric2(const T* xq, const T* xr, int d, int lane, int metric) {
+__device__ __forceinline__ double warp_metric2(const T* xq, double mq, const T* xr, int d, int lane, int metric) {
+  if (metric == 4) return warp_corr2<T>(xq, mq, xr, d, lane);
   return metric == 1 ? warp_cos2<T>(xq, xr, d, lane) : warp_l1sq<T>(xq, xr, d, lane);
 }
 
@@ -206,7 +251,8 @@ struct Refine1Params {
   const int32_t* cand_idx; const float* tau; const float* qn2; float maxrn2; double eps_rel;
   int32_t* st_idx; double* st_val; int32_t* n_keep; double* bw_out; float* lim2_out;
   int32_t* status; int32_t* nzero;
-  int staged;                  // 1: candidate rows are staged through shared memory with cp.async (float32, d % 4 == 0, d <= 128)
+  int staged;                  // 1: candidate rows are staged through shared memory with cp.async (Euclidean sum,
+                               // float32, d % 4 == 0, d <= 128)
 };
 
 template <typename T>
@@ -229,10 +275,12 @@ __global__ void __launch_bounds__(R1_WARPS * 32, 6) refine_topk_kernel(Refine1Pa
   const T* Xr = reinterpret_cast<const T*>(rp.Xr);
   int n_cand = 0;
   bool vec = false;
-  if (rp.metric != 0) {
+  const bool l2sum = euclidean_sum(rp.metric);
+  if (!l2sum) {
+    const double mq = (rp.metric == 4) ? warp_mean<T>(xq, rp.d, lane) : 0.0;
     for (int c0 = 0; c0 < S; ++c0) {
       const int j = p.cand_idx[row * p.cand_stride + c0];
-      const double v = (j >= 0) ? warp_metric2<T>(xq, Xr + (int64_t)j * rp.d, rp.d, lane, rp.metric) : DBL_MAX * 2.0;
+      const double v = (j >= 0) ? warp_metric2<T>(xq, mq, Xr + (int64_t)j * rp.d, rp.d, lane, rp.metric) : DBL_MAX * 2.0;
       if (j >= 0) ++n_cand;
       if (lane == 0) { key[c0] = v; idx[c0] = (j >= 0) ? j : 0x7fffffff; }
     }
@@ -240,7 +288,7 @@ __global__ void __launch_bounds__(R1_WARPS * 32, 6) refine_topk_kernel(Refine1Pa
   if constexpr (sizeof(T) == 4) {
     vec = ((rp.d & 3) == 0) && (((reinterpret_cast<uintptr_t>(rp.Xq) | reinterpret_cast<uintptr_t>(rp.Xr)) & 15) == 0);
   }
-  if (rp.metric != 0) {
+  if (!l2sum) {
     // done above
   } else if (p.staged && sizeof(T) == 4) {
     if constexpr (sizeof(T) == 4) {
@@ -361,6 +409,11 @@ __global__ void __launch_bounds__(R1_WARPS * 32, 6) refine_topk_kernel(Refine1Pa
       }
     }
   }
+  }
+  if (rp.metric == 3) {
+    // sqeuclidean: key = s^2 of the Euclidean sum s (see search2_of_key); +inf padding stays +inf
+    __syncwarp();
+    for (int t = lane; t < S; t += 32) key[t] = key[t] * key[t];
   }
   // 2. sort by (d2, idx); 3. zero-distance count (duplicate detection, graphs.py:787-817)
   const bool small = S <= 32;            // one candidate per lane: both sorts of the row run in registers
@@ -499,10 +552,12 @@ __global__ void __launch_bounds__(R2_THREADS) refine_ball_kernel(Refine2Params p
   const int np2 = next_pow2(L < 2 ? 2 : L);
   const T* xq = reinterpret_cast<const T*>(rp.Xq) + row * rp.d;
   const T* Xr = reinterpret_cast<const T*>(rp.Xr);
+  const double mq = (rp.metric == 4) ? warp_mean<T>(xq, rp.d, lane) : 0.0;
   for (int c = warp; c < L; c += R2_THREADS / 32) {
     int j = p.seg_idx[p0 + c];
-    double d2 = (rp.metric != 0) ? warp_metric2<T>(xq, Xr + (int64_t)j * rp.d, rp.d, lane, rp.metric)
-                                 : warp_dist2<T>(xq, Xr + (int64_t)j * rp.d, rp.d, lane);
+    double d2 = euclidean_sum(rp.metric) ? warp_dist2<T>(xq, Xr + (int64_t)j * rp.d, rp.d, lane)
+                                         : warp_metric2<T>(xq, mq, Xr + (int64_t)j * rp.d, rp.d, lane, rp.metric);
+    if (rp.metric == 3) d2 *= d2;                                  // sqeuclidean: key = s^2, as in stage 1
     if (lane == 0) { key[c] = d2; idx[c] = j; }
   }
   for (int t = L + tid; t < np2; t += R2_THREADS) { key[t] = DBL_MAX * 2.0; idx[t] = 0x7fffffff; }
@@ -622,7 +677,7 @@ extern "C" int gtb_refine_topk(const void* Xq, int64_t nq, const void* Xr, int d
   GTB_CHECK_ARG(nq > 0 && S > 0 && S <= R1_CAP, "S out of range");
   GTB_CHECK_ARG(knn >= 1 && knn <= S, "knn must be in [1, S]");
   GTB_CHECK_ARG(decay < 0 || (thresh > 0 && thresh <= 1), "thresh must be in (0, 1]");
-  GTB_CHECK_ARG(x_kind >= 0 && x_kind <= 5, "x_kind: bit 0 = float64 rows, bits 1-2 = metric (0 euclidean, 1 cosine, 2 cityblock)");
+  GTB_CHECK_ARG(x_kind >= 0 && x_kind <= 9, "x_kind: bit 0 = float64 rows, bits 1-3 = metric (0 euclidean, 1 cosine, 2 cityblock, 3 sqeuclidean, 4 correlation)");
   const int x_is_f64 = x_kind & 1;
   Refine1Params p;
   p.rp = make_row_params(Xq, Xr, d, knn, kmax, decay, thresh, bw_fixed, bw_mode, bw_scale, x_kind >> 1);
@@ -631,7 +686,7 @@ extern "C" int gtb_refine_topk(const void* Xq, int64_t nq, const void* Xr, int d
   p.st_idx = st_idx; p.st_val = st_val; p.n_keep = n_keep; p.bw_out = bw_out; p.lim2_out = lim2_out;
   p.status = status; p.nzero = nzero;
   // float32 rows of whole, 16-byte aligned float4s no longer than one warp-wide load: stage the gathers through smem
-  p.staged = (!x_is_f64 && (x_kind >> 1) == 0 && (d & 3) == 0 && d <= 128 &&
+  p.staged = (!x_is_f64 && euclidean_sum(x_kind >> 1) && (d & 3) == 0 && d <= 128 &&
               (((uintptr_t)Xq | (uintptr_t)Xr) & 15) == 0) ? 1 : 0;
   const size_t smem = p.staged ? (size_t)R1_WARPS * 2 * 8 * d * sizeof(float) : 0;
   if (x_is_f64)
@@ -671,7 +726,7 @@ extern "C" int gtb_refine_ball(const void* Xq, const int32_t* todo_rows, const i
   GTB_CHECK_ARG(nt > 0, "no rows");
   GTB_CHECK_ARG(cap >= 2 && (cap & (cap - 1)) == 0 && cap <= 8192, "cap must be a power of two <= 8192");
   cudaStream_t st = (cudaStream_t)stream;
-  GTB_CHECK_ARG(x_kind >= 0 && x_kind <= 5, "x_kind: bit 0 = float64 rows, bits 1-2 = metric (0 euclidean, 1 cosine, 2 cityblock)");
+  GTB_CHECK_ARG(x_kind >= 0 && x_kind <= 9, "x_kind: bit 0 = float64 rows, bits 1-3 = metric (0 euclidean, 1 cosine, 2 cityblock, 3 sqeuclidean, 4 correlation)");
   const int x_is_f64 = x_kind & 1;
   Refine2Params p;
   p.rp = make_row_params(Xq, Xr, d, knn, kmax, decay, thresh, bw_fixed, bw_mode, bw_scale, x_kind >> 1);

@@ -594,7 +594,9 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
         if (t0 < BIG) thr = t0;
       }
     } else if (MODE == 1) {
-      thr = valid ? (p.lim2[gq] - nx) : -gtb_inf_f();
+      // capped at BIG: every real value stays below it and every padded reference row above it, so a radius wider
+      // than the data (a kernel support beyond all points) cannot admit padded columns j >= nr
+      thr = valid ? fminf(p.lim2[gq] - nx, BIG) : -gtb_inf_f();
     } else {
       thr = 0.f;
     }

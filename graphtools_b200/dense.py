@@ -6,7 +6,7 @@ from . import _engine as E
 from . import pipeline
 
 SYM = {"+": 0, "*": 1, "mnn": 2, None: 3}
-METRIC = {"euclidean": 0, "cosine": 1, "cityblock": 2, "manhattan": 2, "l1": 2}
+METRIC = {"euclidean": 0, "cosine": 1, "cityblock": 2, "manhattan": 2, "l1": 2, "sqeuclidean": 3, "correlation": 4}
 
 
 def _same_dtype(Xq, Xr):
@@ -17,26 +17,46 @@ def _same_dtype(Xq, Xr):
     return Xq.to(dt).contiguous(), Xr.to(dt).contiguous(), int(is64)
 
 
+def _row_centred(X):
+    """float64 copy of X minus each row's mean, scipy's correlation arithmetic (``XA - XA.mean(axis=1)``, then its
+    cosine routine).  Constant rows are set to exactly zero, so that their distances are NaN whatever the rounding of
+    their mean: the degenerate rows of ``pipeline.degenerate_rows``."""
+    X = X.to(torch.float64)
+    C = X - X.mean(dim=1, keepdim=True)
+    C[pipeline.degenerate_rows(X, "correlation")] = 0.0
+    return C.contiguous()
+
+
+def _operands(Xq, Xr, metric):
+    """(Xq, Xr, is64, metric code) for gtb_dense_kernel: correlation runs the cosine branch on row-centred float64
+    copies (8 n d bytes each, small beside the n^2 output)."""
+    Xq, Xr, is64 = _same_dtype(Xq, Xr)
+    if metric != "correlation":
+        return Xq, Xr, is64, METRIC[metric]
+    Cq = _row_centred(Xq)
+    return Cq, (Cq if Xr is Xq else _row_centred(Xr)), 1, METRIC["cosine"]
+
+
 def dense_affinity(Xq, Xr, bw_q, bw_r, decay, thresh, symm=None, theta=None, want_rowsum=True, metric="euclidean"):
     """[nq, nr] float64 thresholded alpha-decay affinities; symmetrised in the same sweep when
     ``bw_r`` is given (square problems)."""
-    Xq, Xr, is64 = _same_dtype(Xq, Xr)
+    Xq, Xr, is64, code = _operands(Xq, Xr, metric)
     nq, d = Xq.shape
     nr = Xr.shape[0]
     out = pipeline._empty((nq, nr), torch.float64)
     rowsum = pipeline._empty((nq,), torch.float64) if want_rowsum else None
     what = 2 if bw_r is not None else 1
-    E.call("gtb_dense_kernel", Xq, nq, Xr, nr, d, is64, what, METRIC[metric], bw_q, bw_r, float(decay), float(thresh),
+    E.call("gtb_dense_kernel", Xq, nq, Xr, nr, d, is64, what, code, bw_q, bw_r, float(decay), float(thresh),
            SYM[symm], 0.0 if theta is None else float(theta), out, rowsum)
     return out, rowsum
 
 
 def dense_distances(Xq, Xr, metric="euclidean"):
-    Xq, Xr, is64 = _same_dtype(Xq, Xr)
+    Xq, Xr, is64, code = _operands(Xq, Xr, metric)
     nq, d = Xq.shape
     nr = Xr.shape[0]
     out = pipeline._empty((nq, nr), torch.float64)
-    E.call("gtb_dense_kernel", Xq, nq, Xr, nr, d, is64, 0, METRIC[metric], None, None, 0.0, 0.0, 3, 0.0, out, None)
+    E.call("gtb_dense_kernel", Xq, nq, Xr, nr, d, is64, 0, code, None, None, 0.0, 0.0, 3, 0.0, out, None)
     return out
 
 

@@ -43,10 +43,8 @@ class TraditionalGraph(DataGraph):
                     precomputed, data.shape))
             elif (data < 0).sum() > 0:
                 raise ValueError("Precomputed {} should be non-negative".format(precomputed))
-        if precomputed is None and distance not in ("euclidean", "cosine", "cityblock", "manhattan", "l1"):
-            raise NotImplementedError(
-                "graphtools_b200 accelerates the euclidean, cosine and cityblock metrics (got distance={!r})".format(
-                    distance))
+        if precomputed is None and distance not in pipeline.METRIC_NAMES:
+            raise NotImplementedError(pipeline.unsupported_metric_message(distance))
         self.knn = knn
         self.decay = decay
         self.bandwidth = bandwidth
@@ -95,22 +93,20 @@ class TraditionalGraph(DataGraph):
             self._dev_X = self._dense_f32(self.data_nu)
         return self._dev_X
 
-    def _zero_rows(self, X):
-        """Rows of ``X`` that are all zero, for the cosine metric (None otherwise): scipy's cosine distance from such
-        a row is NaN."""
-        if self._metric() != "cosine":
-            return None
-        return (X == 0).all(dim=1)
+    def _degenerate_rows(self, X):
+        """Rows of ``X`` from which scipy's distance is NaN (None for metrics without such rows): all-zero rows under
+        cosine, constant rows under correlation."""
+        return pipeline.degenerate_rows(X, self._metric())
 
     def _adaptive_bandwidth(self, Xq_op, ref_op, knn_eff):
         """Distance to the knn_eff-th nearest reference point (self counted when in-sample):
         np.partition(pdx, k)[:, :k].max (graphs.py:1583-1587, :1655-1656).
 
-        Cosine with all-zero rows: their distances are NaN in the reference, which np.partition sorts last. So the
-        neighbours are searched among the non-zero reference rows, and the bandwidth is NaN where the k smallest
-        entries of a row include a NaN: every zero query row, and every row when fewer than k reference rows are
-        non-zero."""
-        zq, zr = self._zero_rows(Xq_op.X), self._zero_rows(ref_op.X)
+        Degenerate rows (all-zero under cosine, constant under correlation): their distances are NaN in the
+        reference, which np.partition sorts last. So the neighbours are searched among the other reference rows, and
+        the bandwidth is NaN where the k smallest entries of a row include a NaN: every degenerate query row, and
+        every row when fewer than k reference rows are not degenerate."""
+        zq, zr = self._degenerate_rows(Xq_op.X), self._degenerate_rows(ref_op.X)
         if zq is None or not bool(zq.any().item() or zr.any().item()):
             _, info = pipeline.knn_kernel(None, ref_op, Xq_op, knn=knn_eff, decay=max(float(self.decay), 1.0),
                                           thresh=0.5, bandwidth_scale=1.0)
@@ -118,8 +114,8 @@ class TraditionalGraph(DataGraph):
         bw = torch.full((Xq_op.n,), float("nan"), dtype=torch.float64, device=Xq_op.X.device)
         keep_r, keep_q = (~zr).nonzero().flatten(), (~zq).nonzero().flatten()
         if keep_r.shape[0] >= knn_eff and keep_q.shape[0] > 0:
-            ref_nz = pipeline.SearchOperand(ref_op.X[keep_r].contiguous(), metric="cosine")
-            qry_nz = pipeline.SearchOperand(Xq_op.X[keep_q].contiguous(), mean=ref_nz.mean, metric="cosine")
+            ref_nz = pipeline.SearchOperand(ref_op.X[keep_r].contiguous(), metric=self._metric())
+            qry_nz = pipeline.SearchOperand(Xq_op.X[keep_q].contiguous(), mean=ref_nz.mean, metric=self._metric())
             _, info = pipeline.knn_kernel(None, ref_nz, qry_nz, knn=knn_eff, decay=max(float(self.decay), 1.0),
                                           thresh=0.5, bandwidth_scale=1.0)
             bw[keep_q] = info["bandwidth"]
@@ -164,8 +160,9 @@ class TraditionalGraph(DataGraph):
         if not (self.thresh is not None and self.thresh > 0 and self.decay is not None
                 and not callable(self.bandwidth) and self.knn is not None and self.knn + 1 + 8 <= 128):
             return False
-        # a zero row under the cosine metric has NaN distances, i.e. affinity 1 to every sample: not sparse
-        zero = self._zero_rows(self._X())
+        # a degenerate row (all-zero under cosine, constant under correlation) has NaN distances, i.e. affinity 1 to
+        # every sample: not sparse
+        zero = self._degenerate_rows(self._X())
         return zero is None or not bool(zero.any().item())
 
     def _build_kernel_via_sparse(self):

@@ -71,6 +71,16 @@ def _splice_rows(R, rows, R2):
     return pipeline.DeviceCSR(indptr, idx, val, R.shape)
 
 
+def _zero_distance_pairs(X, rows, metric):
+    """{(j, i)}: every sample j < i at distance exactly 0 from row i, for each i in ``rows`` (the rows with more than one
+    zero-distance candidate) -- the pairs the reference names from its neighbour indices (graphs.py:787-817).  Under
+    correlation these include affine copies a x + b (a > 0), which are not equal rows."""
+    import torch
+    from . import dense
+    D = dense.dense_distances(X[torch.from_numpy(rows).to(X.device)], X, metric)
+    return {(int(j), int(rows[r])) for r, j in (D == 0).nonzero().cpu().tolist() if j < rows[r]}
+
+
 class kNNGraph(DataGraph):
     """K nearest neighbours graph, optionally with alpha-decay affinities."""
 
@@ -102,10 +112,8 @@ class kNNGraph(DataGraph):
         if n_pca in [None, 0, False] and data.shape[1] > 500:
             warnings.warn("Building a kNNGraph on data of shape {} is "
                           "expensive. Consider setting n_pca.".format(data.shape), UserWarning)
-        if distance not in ("euclidean", "cosine", "cityblock", "manhattan", "l1"):
-            raise NotImplementedError(
-                "graphtools_b200 accelerates the euclidean, cosine and cityblock metrics (got distance={!r})".format(
-                    distance))
+        if distance not in pipeline.METRIC_NAMES:
+            raise NotImplementedError(pipeline.unsupported_metric_message(distance))
         self.knn = knn
         self.knn_max = knn_max
         self.search_multiplier = search_multiplier
@@ -151,7 +159,9 @@ class kNNGraph(DataGraph):
         (centred k-major copy + norms).  Stands in for the reference's sklearn NearestNeighbors
         (graphs.py:748-769)."""
         if "_ref_operand" not in self.__dict__:
-            self._ref_operand = pipeline.SearchOperand(self._reference_rows(), metric=self.distance)
+            rows = self._reference_rows()
+            pipeline.reject_constant_rows(rows, self.distance)
+            self._ref_operand = pipeline.SearchOperand(rows, metric=self.distance)
         return self._ref_operand
 
     def _reference_rows(self):
@@ -331,15 +341,20 @@ class kNNGraph(DataGraph):
         if n_dup_rows == 0:
             return
         total = int((nzero - 1).clamp(min=0).sum().item())
+        pairs = None
         if total < 20 and qry is ref:
             rows = (nzero > 1).nonzero().flatten().cpu().numpy()
-            Xh = ref.X.cpu().numpy()
-            pairs = set()
-            for i in rows:
-                same = np.flatnonzero((Xh == Xh[i]).all(axis=1))
-                for j in same:
-                    if j < i:
-                        pairs.add((int(j), int(i)))
+            if ref.metric in ("sqeuclidean", "correlation"):
+                pairs = _zero_distance_pairs(ref.X, rows, ref.metric) or None
+            else:
+                Xh = ref.X.cpu().numpy()
+                pairs = set()
+                for i in rows:
+                    same = np.flatnonzero((Xh == Xh[i]).all(axis=1))
+                    for j in same:
+                        if j < i:
+                            pairs.add((int(j), int(i)))
+        if pairs is not None:
             names = ", ".join("{} and {}".format(a, b) for a, b in sorted(pairs))
             warnings.warn("Detected zero distance between samples {}. Consider removing duplicates to avoid "
                           "errors in downstream processing.".format(names), RuntimeWarning)
@@ -363,6 +378,7 @@ class kNNGraph(DataGraph):
         from . import distributed as gd
         with _logger.log_task("KNN search"):
             Yd = self._dense_f32(Y).to(ref.X.dtype)
+            pipeline.reject_constant_rows(Yd, ref.metric)
             if gd.active() and np.ndim(bandwidth) == 0 and Yd.shape[0] >= gd.MIN_ROWS_PER_RANK * gd.world_size():
                 return self._kernel_to_data_sharded(Yd, ref, knn, knn_max, bandwidth, bandwidth_scale)
             qry = pipeline.SearchOperand(Yd, mean=ref.mean, metric=ref.metric)

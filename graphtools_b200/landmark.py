@@ -125,6 +125,7 @@ class LandmarkGraph(DataGraph):
         data = self.data if not hasattr(self, "data_nu") else self.data_nu
         X = self._dense_f32(data)
         metric = getattr(self, "distance", "euclidean")          # cdist(..., metric=self.distance), graphs.py:1212
+        pipeline.reject_constant_rows(X, metric)
         ref = pipeline.SearchOperand(X[torch.from_numpy(landmark_indices).to(X.device)].contiguous(), metric=metric)
         qry = pipeline.SearchOperand(X, mean=ref.mean, metric=metric)
         nearest, _ = pipeline.knn_kernel(None, ref, qry, knn=1, decay=None)   # exact float64 argmin per sample

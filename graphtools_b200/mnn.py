@@ -75,6 +75,7 @@ class MNNGraph(DataGraph):
     def build_kernel(self):
         """Assemble the batch-block kernel on the device (graphs.py:1857-1936)."""
         from .factory import Graph
+        pipeline.reject_constant_rows(self.data_nu, self.distance)
         dev = pipeline._dev()
         sample_idx = np.asarray(self.sample_idx)
         n = self.data_nu.shape[0]

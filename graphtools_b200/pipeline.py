@@ -15,7 +15,8 @@ from . import _engine as E
 
 SYM_MODES = {"+": 0, "*": 1, "mnn": 2, None: 3}
 METRIC_ALIASES = {"manhattan": "cityblock", "l1": "cityblock", "l2": "euclidean"}
-METRIC_CODE = {"euclidean": 0, "cosine": 1, "cityblock": 2}
+METRIC_CODE = {"euclidean": 0, "cosine": 1, "cityblock": 2, "sqeuclidean": 3, "correlation": 4}
+METRIC_NAMES = tuple(METRIC_CODE) + ("manhattan", "l1")      # the ``distance`` values graphs accept
 AUTO_TC = "tch1"         # tensor-core flavour picked by impl="auto": "tch1" (fp16, one product, seeded), "tch" (fp16x2), "tc16" (bf16x3) or "tc" (3xTF32)
 BALL_CAP = 8192          # longest radius-pass row handled by refine_ball (shared-memory sort)
 _STATS = {}
@@ -23,6 +24,41 @@ _STATS = {}
 
 class RowTooLong(NotImplementedError):
     """A row has more neighbours inside the kernel radius than the radius-pass refine handles (BALL_CAP)."""
+
+
+def unsupported_metric_message(distance):
+    return ("graphtools_b200 accelerates the euclidean, cosine and cityblock metrics, and sqeuclidean and correlation "
+            "(got distance={!r})".format(distance))
+
+
+def degenerate_rows(X, metric):
+    """Rows on which ``metric`` has no value (scipy's distances from them are NaN): all-zero rows under cosine, constant
+    rows (max == min, whose centred row is zero) under correlation; None for the other metrics.  ``X``: torch tensor
+    or numpy array [n, d] (also a scipy sparse matrix under correlation); the mask is a bool tensor or numpy array."""
+    if metric == "cosine":
+        return (X == 0).all(1)
+    if metric == "correlation":
+        if isinstance(X, torch.Tensor):
+            return X.amax(dim=1) == X.amin(dim=1)
+        hi, lo = X.max(axis=1), X.min(axis=1)
+        if not isinstance(X, np.ndarray):                   # scipy sparse: matrices of shape [n, 1]
+            hi, lo = hi.toarray(), lo.toarray()
+        return np.asarray(hi == lo).reshape(-1)
+    return None
+
+
+def reject_constant_rows(X, metric):
+    """Searches under correlation (kNN, MNN and landmark graphs, out-of-sample kernels) raise ValueError on constant
+    rows before any work: the reference's neighbours of such a row are in undefined order, and its symmetrised kernel
+    spreads their NaN distances into other rows.  (Exact graphs accept them: their affinity is 1.)"""
+    if metric != "correlation":
+        return
+    n = int(degenerate_rows(X, metric).sum())
+    if n:
+        raise ValueError(
+            "{} of {} rows are constant: their correlation distance to every row is undefined (the row minus its mean "
+            "is zero). Remove them, or use graphtype='exact', which gives them affinity 1 to every "
+            "sample.".format(n, X.shape[0]))
 
 
 def stats():
@@ -161,7 +197,13 @@ class SearchOperand:
         rounded once), on which squared Euclidean distance = 2 x cosine distance; the exact stage evaluates
         1 - x.y / (|x||y|) on the original rows.  All-zero rows stay zero, as in sklearn's ``normalize``; their
         search distance to a normalised row is 1 (to another zero row 0), below the 2 x 1 of their exact cosine
-        distance, so the certification bounds stay conservative for them."""
+        distance, so the certification bounds stay conservative for them.
+
+        metric="correlation": as cosine, after subtracting each row's own mean in float64 (scipy centres every row
+        by its np.mean before its cosine routine): row-centred, normalised, column-centred, rounded once.  ``X``
+        keeps the original rows, which the exact stage and the reference's Euclidean fallback read.
+
+        metric="sqeuclidean": the Euclidean operand, unchanged; the exact stage squares the Euclidean distance."""
         n, d = X.shape
         self.X, self.n, self.d = X, n, d
         self.metric = metric
@@ -170,7 +212,7 @@ class SearchOperand:
         self.d_pad = (d + 7) // 8 * 8
         metric = METRIC_ALIASES.get(metric, metric)
         self.metric = metric
-        if metric not in ("euclidean", "cosine", "cityblock"):
+        if metric not in METRIC_CODE:
             raise NotImplementedError("metric {!r} is not supported by the CUDA search".format(metric))
         if metric == "cityblock":
             # |x - y| is translation invariant and has no GEMM form: the search copy is the float32 data itself,
@@ -179,9 +221,11 @@ class SearchOperand:
             self.Xs = X.to(torch.float32).contiguous() if self.is64 else X
             self._kmean = None
             mean = torch.zeros((d,), dtype=torch.float32, device=X.device) if mean is None else mean
-        elif self.is64 or metric == "cosine":
+        elif self.is64 or metric in ("cosine", "correlation"):
             rows = X.to(torch.float64)
-            if metric == "cosine":
+            if metric == "correlation":
+                rows = rows - rows.mean(dim=1, keepdim=True)
+            if metric in ("cosine", "correlation"):
                 norms = rows.norm(dim=1, keepdim=True)
                 rows = rows / torch.where(norms > 0, norms, torch.ones_like(norms))
             if mean is None:

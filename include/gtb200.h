@@ -124,10 +124,13 @@ int gtb_knn_radius_tc(const void* q_hi, const void* q_lo, const float* qn2, cons
 /* ---- K3 float64 re-evaluation, bandwidth, affinities, CSR emission: replaces graphs.py:886-911
  * and _build_csr_from_neighbors (graphs.py:450-559) ------------------------------------------ */
 /* Xq / Xr are the ORIGINAL rows used for the exact distances; x_kind bit 0: rows are float64 (e.g. PCA output)
- * instead of float32; bits 1-2: metric -- 1 = cosine: exact distances 1 - x.y/(|x||y|) (sklearn cosine_distances, the
+ * instead of float32; bits 1-3: metric -- 1 = cosine: exact distances 1 - x.y/(|x||y|) (sklearn cosine_distances, the
  * metric behind knn_tree for distance="cosine", graphs.py:763-768) while the fast pass ran on the row-normalised
  * copies, where |x^ - y^|^2 = 2 d_cos; 2 = cityblock: exact sum |x - y|, fast pass = gtb_knn_topk_simt_l1 (tau is a
- * distance, the rounding bound is eps_rel * tau, qn2 / maxrn2 carry L1 norms for float64 inputs or NULL / 0).  decay < 0 means binary kNN (decay=None); kmax <= 0 means knn_max=None;
+ * distance, the rounding bound is eps_rel * tau, qn2 / maxrn2 carry L1 norms for float64 inputs or NULL / 0); 3 =
+ * sqeuclidean: exact sum (x - y)^2 on the Euclidean fast pass and operands (radii in squared units); 4 = correlation:
+ * cosine of the rows centred by their own float64 means, fast pass on the row-centred, row-normalised copies as for
+ * cosine.  decay < 0 means binary kNN (decay=None); kmax <= 0 means knn_max=None;
  * bw_mode 0: bandwidth = distance to the knn-th candidate (graphs.py:892), 1: scalar bw_fixed[0],
  * 2: per-row bw_fixed[nq].  cand_idx rows are cand_stride apart (first S entries used); tau holds ntau
  * thresholds per row (lists built over disjoint reference subsets), the row's bound is their minimum.  status: 1 done, 0 needs radius pass, 2 needs radius pass and its
@@ -247,8 +250,9 @@ int gtb_landmark_op(const int64_t* ptr, const int32_t* lab, const double* raw, c
  * what pdist / cdist compute).  what 0: out = distances; 1: out = thresholded affinities exp(-(d/bw_q[i])^decay);
  * 2: additionally symmetrised with the transposed entry (symm 0 '+', 1 '*', 2 'mnn', 3 none);
  * rowsum (optional) receives the row L1 sums (a separate deterministic pass).  metric 0: Euclidean distances;
- * 1: cosine distances 1 - x.y/(|x||y|) with |cos| clamped to 1; 2: cityblock (scipy pdist / cdist, graphs.py:1552,
- * :1653) */
+ * 1: cosine distances 1 - x.y/(|x||y|) with |cos| clamped to 1; 2: cityblock; 3: sqeuclidean (scipy pdist / cdist,
+ * graphs.py:1552, :1653).  Correlation distances are metric 1 on rows centred by their float64 means, as scipy computes
+ * them. */
 int gtb_dense_kernel(const void* Xq, int64_t nq, const void* Xr, int64_t nr, int d, int x_is_f64, int what, int metric,
                      const double* bw_q, const double* bw_r, double decay, double thresh, int symm, double theta,
                      double* out, double* rowsum, void* stream);
