@@ -43,7 +43,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 namespace {
 
@@ -1160,9 +1159,10 @@ extern "C" int gtb_row_norms(const float* X, int64_t n, int d, const float* mean
 // largest scaled squared norm the fp16 flavour accepts: scale^2 * max|row|^2 must stay <= this
 extern "C" float gtb_tc_fp16_maxnorm(void) { return TC_H_MAXNORM; }
 
-extern "C" int gtb_prepare_operand_tc(const float* X, int64_t n, int d, const float* mean, int role, void* hi,
-                                      void* lo, int64_t n_pad, int Kp, int dtype, float scale, float* norm2,
-                                      float* maxnorm, void* stream) {
+// Argument checks and the split into hi/lo pairs of `dtype`, shared by gtb_prepare_operand_tc and gtb_split_operand_tc;
+// with `norms`, the squared norms (and their maximum) are computed first, into norm2
+static int tc_operand(const float* X, int64_t n, int d, const float* mean, int role, void* hi, void* lo, int64_t n_pad,
+                      int Kp, int dtype, float scale, float* norm2, float* maxnorm, bool norms, cudaStream_t st) {
   GTB_CHECK_ARG(n > 0 && d > 0 && n_pad >= n && n_pad % 128 == 0, "bad shape");
   GTB_CHECK_ARG(dtype >= 0 && dtype <= 2, "dtype must be 0 (tf32 pairs in float32), 1 (bfloat16 pairs) or 2 (float16 pairs)");
   const int epk = dtype ? 16 : 8;
@@ -1170,10 +1170,11 @@ extern "C" int gtb_prepare_operand_tc(const float* X, int64_t n, int d, const fl
                 "Kp must be a multiple of 8 (tf32, <= 104) / 16 (bf16 <= 128, fp16 <= 512) and >= d+1 (fp16: d+2)");
   GTB_CHECK_ARG(role == 0 || role == 1, "role must be 0 (query) or 1 (reference)");
   GTB_CHECK_ARG(dtype != 2 || scale > 0.f, "the fp16 flavour needs a positive scale");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (maxnorm) GTB_CUDA(cudaMemsetAsync(maxnorm, 0, sizeof(float), st));
-  tc_norms_kernel<<<(unsigned)gtb_cdiv(n_pad * 32, 256), 256, 0, st>>>(X, n, d, mean, n_pad, norm2, maxnorm);
-  GTB_CHECK_LAUNCH();
+  if (norms) {
+    if (maxnorm) GTB_CUDA(cudaMemsetAsync(maxnorm, 0, sizeof(float), st));
+    tc_norms_kernel<<<(unsigned)gtb_cdiv(n_pad * 32, 256), 256, 0, st>>>(X, n, d, mean, n_pad, norm2, maxnorm);
+    GTB_CHECK_LAUNCH();
+  }
   if (dtype == 0)
     tc_split_kernel<<<(unsigned)gtb_cdiv(n_pad * Kp, 256), 256, 0, st>>>(X, n, d, mean, role, norm2, n_pad, Kp,
                                                                         (float*)hi, (float*)lo);
@@ -1187,30 +1188,19 @@ extern "C" int gtb_prepare_operand_tc(const float* X, int64_t n, int d, const fl
   return GTB_OK;
 }
 
+extern "C" int gtb_prepare_operand_tc(const float* X, int64_t n, int d, const float* mean, int role, void* hi,
+                                      void* lo, int64_t n_pad, int Kp, int dtype, float scale, float* norm2,
+                                      float* maxnorm, void* stream) {
+  return tc_operand(X, n, d, mean, role, hi, lo, n_pad, Kp, dtype, scale, norm2, maxnorm, true, (cudaStream_t)stream);
+}
+
 // The split alone, from norms that are already on hand (gtb_row_norms): both roles of an in-sample build share one pass
 // over the norms instead of recomputing them per role
 extern "C" int gtb_split_operand_tc(const float* X, int64_t n, int d, const float* mean, int role, void* hi, void* lo,
                                     int64_t n_pad, int Kp, int dtype, float scale, const float* norm2, void* stream) {
-  GTB_CHECK_ARG(n > 0 && d > 0 && n_pad >= n && n_pad % 128 == 0, "bad shape");
-  GTB_CHECK_ARG(dtype >= 0 && dtype <= 2, "dtype must be 0 (tf32 pairs in float32), 1 (bfloat16 pairs) or 2 (float16 pairs)");
-  const int epk = dtype ? 16 : 8;
-  GTB_CHECK_ARG(Kp % epk == 0 && Kp >= d + 1 + (dtype == 2) && Kp / epk <= (dtype == 2 ? 32 : (dtype ? 8 : 13)),
-                "Kp must be a multiple of 8 (tf32, <= 104) / 16 (bf16 <= 128, fp16 <= 512) and >= d+1 (fp16: d+2)");
-  GTB_CHECK_ARG(role == 0 || role == 1, "role must be 0 (query) or 1 (reference)");
-  GTB_CHECK_ARG(dtype != 2 || scale > 0.f, "the fp16 flavour needs a positive scale");
   GTB_CHECK_ARG(norm2 != nullptr, "norm2 (from gtb_row_norms) is required");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (dtype == 0)
-    tc_split_kernel<<<(unsigned)gtb_cdiv(n_pad * Kp, 256), 256, 0, st>>>(X, n, d, mean, role, norm2, n_pad, Kp,
-                                                                        (float*)hi, (float*)lo);
-  else if (dtype == 1)
-    tc_split16_kernel<<<(unsigned)gtb_cdiv(n_pad * Kp, 256), 256, 0, st>>>(X, n, d, mean, role, norm2, n_pad, Kp,
-                                                                          (__nv_bfloat16*)hi, (__nv_bfloat16*)lo);
-  else
-    tc_split16h_kernel<<<(unsigned)gtb_cdiv(n_pad * Kp, 256), 256, 0, st>>>(X, n, d, mean, role, norm2, n_pad, Kp, scale,
-                                                                           (__half*)hi, (__half*)lo);
-  GTB_CHECK_LAUNCH();
-  return GTB_OK;
+  return tc_operand(X, n, d, mean, role, hi, lo, n_pad, Kp, dtype, scale, const_cast<float*>(norm2), nullptr, false,
+                    (cudaStream_t)stream);
 }
 
 // candidate buffers of every row + the piece buffers and piece records of a split last round
@@ -1241,9 +1231,6 @@ extern "C" int gtb_knn_topk_tc_seeded(const void* q_hi, const void* q_lo, const 
   p.cand_idx = cand_idx; p.cand_buf = reinterpret_cast<uint2*>(scratch); p.tau = tau; p.sync_ctr = pace;
   p.seed_tau = seed_tau; p.tile_stride = tile_stride;
   p.piece_buf = p.cand_buf + nq_pad * TC_GROUPS * TC_CAP;   // second part of the scratch (gtb_tc_scratch_bytes)
-  if (const char* e = getenv("GTB_TC_SPLIT")) {              // kernel experiments: 0 = never split the last round
-    if (atoi(e) == 0) p.piece_buf = nullptr;
-  }
   return launch_tc<0>(q_hi, q_lo, r_hi, r_lo, Kp, dtype, list, cluster, qtiles, p, (cudaStream_t)stream);
 }
 

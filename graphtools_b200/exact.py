@@ -108,7 +108,7 @@ class TraditionalGraph(DataGraph):
         every row when fewer than k reference rows are not degenerate."""
         zq, zr = self._degenerate_rows(Xq_op.X), self._degenerate_rows(ref_op.X)
         if zq is None or not bool(zq.any().item() or zr.any().item()):
-            _, info = pipeline.knn_kernel(None, ref_op, Xq_op, knn=knn_eff, decay=max(float(self.decay), 1.0),
+            _, info = pipeline.knn_kernel(ref_op, Xq_op, knn=knn_eff, decay=max(float(self.decay), 1.0),
                                           thresh=0.5, bandwidth_scale=1.0)
             return info["bandwidth"]
         bw = torch.full((Xq_op.n,), float("nan"), dtype=torch.float64, device=Xq_op.X.device)
@@ -116,7 +116,7 @@ class TraditionalGraph(DataGraph):
         if keep_r.shape[0] >= knn_eff and keep_q.shape[0] > 0:
             ref_nz = pipeline.SearchOperand(ref_op.X[keep_r].contiguous(), metric=self._metric())
             qry_nz = pipeline.SearchOperand(Xq_op.X[keep_q].contiguous(), mean=ref_nz.mean, metric=self._metric())
-            _, info = pipeline.knn_kernel(None, ref_nz, qry_nz, knn=knn_eff, decay=max(float(self.decay), 1.0),
+            _, info = pipeline.knn_kernel(ref_nz, qry_nz, knn=knn_eff, decay=max(float(self.decay), 1.0),
                                           thresh=0.5, bandwidth_scale=1.0)
             bw[keep_q] = info["bandwidth"]
         return bw
@@ -170,7 +170,7 @@ class TraditionalGraph(DataGraph):
         X = self._X()
         n = X.shape[0]
         op = pipeline.SearchOperand(X, metric=self._metric())
-        R, info = pipeline.knn_kernel(None, op, op, knn=self.knn + 1, knn_max=None, decay=self.decay,
+        R, info = pipeline.knn_kernel(op, op, knn=self.knn + 1, knn_max=None, decay=self.decay,
                                       thresh=self.thresh, bandwidth=self.bandwidth,
                                       bandwidth_scale=self.bandwidth_scale)
         self._dev_bandwidth = info["bandwidth"]

@@ -284,8 +284,8 @@ class kNNGraph(DataGraph):
         """Raw kernel rows of ``qry`` against ``ref``.  ``nq_total``: the query rows are this rank's shard of that
         many rows (the search schedule is then replayed on counts summed over the ranks)."""
         if self.decay is None or self.thresh == 1:
-            return pipeline.knn_kernel(None, ref, qry, knn=knn, knn_max=None, decay=None)
-        R, info = pipeline.knn_kernel(None, ref, qry, knn=knn, knn_max=knn_max, decay=self.decay,
+            return pipeline.knn_kernel(ref, qry, knn=knn, knn_max=None, decay=None)
+        R, info = pipeline.knn_kernel(ref, qry, knn=knn, knn_max=knn_max, decay=self.decay,
                                       thresh=self.thresh, bandwidth=bandwidth, bandwidth_scale=bandwidth_scale)
         if ref.metric != "euclidean":
             R = self._euclidean_fallback(R, info, qry, ref, knn, knn_max, nq_total)
@@ -326,7 +326,7 @@ class kNNGraph(DataGraph):
         sub = pipeline.SearchOperand(qry.X[rows].contiguous(), mean=eref.mean, metric="euclidean")
         bw = info["bandwidth"][rows].cpu().numpy()
         kmax = ref.n if knn_max is None else knn_max
-        R2, _ = pipeline.knn_kernel(None, eref, sub, knn=knn, knn_max=kmax if s_final == kmax else None,
+        R2, _ = pipeline.knn_kernel(eref, sub, knn=knn, knn_max=kmax if s_final == kmax else None,
                                     decay=self.decay, thresh=self.thresh, bandwidth=bw, bandwidth_scale=1.0)
         pipeline._STATS.clear()
         pipeline._STATS.update(main_stats)           # stats() describes the metric search, plus the rebuilt rows

@@ -128,7 +128,7 @@ class LandmarkGraph(DataGraph):
         pipeline.reject_constant_rows(X, metric)
         ref = pipeline.SearchOperand(X[torch.from_numpy(landmark_indices).to(X.device)].contiguous(), metric=metric)
         qry = pipeline.SearchOperand(X, mean=ref.mean, metric=metric)
-        nearest, _ = pipeline.knn_kernel(None, ref, qry, knn=1, decay=None)   # exact float64 argmin per sample
+        nearest, _ = pipeline.knn_kernel(ref, qry, knn=1, decay=None)   # exact float64 argmin per sample
         return nearest.indices.cpu().numpy().astype(np.int64)
 
     def _spectral_impl(self):

@@ -7,6 +7,8 @@ Everything stays in HBM as torch tensors; the two host synchronisations per kern
 reads of `number of uncertified rows` and `nnz` (sizes of the next allocations).
 """
 import math
+from collections import namedtuple
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -267,27 +269,10 @@ class SearchOperand:
     def n2(self):
         return self.simt()[1]
 
-    # -- tensor-core operand: row-major [n_pad][Kp] hi/lo pair for one role (0 query, 1 reference);
-    #    dtype 0 = tf32 pairs stored as float32 (3xTF32), dtype 1 = bfloat16 pairs (bf16x3)
+    # -- tensor-core operand: row-major [n_pad][Kp] hi/lo pair for one role (0 query, 1 reference) in the layout of
+    #    one flavour's dtype code (TC_FLAVOURS)
     def kp(self, dtype=0):
-        # rows are whole 32-byte k-steps (16 bf16 / 8 tf32 elements): SWIZZLE_128B blocks plus SWIZZLE_32B
-        # tail blocks.  (Padding bf16 rows to whole 128-byte blocks was measured slower: 699 vs 682 ms at
-        # d = 100 -- the extra MMAs cost more than the tail blocks.)
-        import os
-        step = 16 if dtype else 8
-        step = int(os.environ.get("GTB_KP_STEP", step))      # experiments: 64 (bf16) / 32 (tf32) = whole 128-byte blocks
-        # float16 operands keep one more column: the low part of |y|^2 (shared by the two- and one-product flavours)
-        return (self.d + 1 + (1 if dtype >= 2 else 0) + step - 1) // step * step
-
-    @property
-    def Kp(self):
-        return self.kp(0)
-
-    def tc_ok(self, dtype=0):
-        if self.metric == "cityblock":
-            return False                                  # no GEMM form: CUDA-core L1 kernel only
-        # resident query tile: 13 tf32 / 8 bf16 k-steps; the fp16x2 flavour streams longer rows in chunks (d <= 510)
-        return self.kp(dtype) // (16 if dtype else 8) <= {0: 13, 1: 8, 2: 32, 3: 8}[dtype]
+        return TC_FLAVOURS[dtype].kp(self.d)
 
     def l1_norms(self):
         """(per-row L1 norms float32 [n], max) of the search copy -- bound on its rounding for float64 inputs."""
@@ -298,8 +283,8 @@ class SearchOperand:
 
     def tc(self, role, dtype=0, scale=1.0):
         """(hi, lo, norm2) of one role; dtype 0 = tf32 pairs in float32, 1 = bfloat16 pairs, 2 = float16 pairs of the
-        data scaled by ``scale`` (norm2 stays unscaled)."""
-        dtype = min(dtype, 2)                             # the one-product flavour reads the fp16x2 hi arrays
+        data scaled by ``scale`` (norm2 stays unscaled); 3 = the float16 pairs of dtype 2."""
+        dtype = TC_FLAVOURS[dtype].operand
         key = (role, dtype, float(scale))
         if key not in self._tc:
             Kp = self.kp(dtype)
@@ -422,24 +407,6 @@ def choose_S(knn_eff, binary):
         "knn={} needs a candidate list longer than 128; not supported by the fused top-k yet".format(knn_eff))
 
 
-def seed_stride():
-    """GTB_TC_SEED_STRIDE: the seed sweep of the one-product flavour visits every stride-th reference tile (1 = off)."""
-    import os
-    return int(os.environ.get("GTB_TC_SEED_STRIDE", "16"))
-
-
-def seedable(ref):
-    """A strided sample needs enough tiles to carry the order statistic: 32 sampled tiles at least."""
-    st = seed_stride()
-    return st > 1 and ref.n_pad // 128 >= 32 * st
-
-
-def tc_cluster():
-    """GTB_TC_CLUSTER = 1 | 2 | 4: CTAs per cluster sharing each reference tile by TMA multicast."""
-    import os
-    return int(os.environ.get("GTB_TC_CLUSTER", "2"))
-
-
 def default_impl():
     """GTB_SEARCH_IMPL = tc (3xTF32 tensor cores) | tc16 (bf16x3 tensor cores) | tch (fp16x2 tensor cores: two
     products, wider certified bound) | tch1 (fp16, ONE product, seeded thresholds, lists of 64) | simt (fp32 CUDA
@@ -483,9 +450,6 @@ def fp16_scale(maxnorm):
     return 2.0 ** math.floor(0.5 * math.log2(limit / maxnorm))
 
 
-TC_DTYPE = {"tc": 0, "tc16": 1, "tch": 2, "tch1": 3}
-
-
 def eps_rel_tch1(d):
     """fp16x1 (A_hi B_hi only, float16): both operands are rounded to 11 bits, |delta(2 x.y)| <= 2 (2 u + u^2)
     sum |x_k||y_k| <= 2^-10 (1 + 2^-12) (|x~|^2 + |y~|^2) with u = 2^-11; |y|^2 keeps 22 bits (hi + spare-column low
@@ -499,9 +463,192 @@ def eps_rel_simt(d):
     return 2.0 * (d + 16) * 2.0 ** -24
 
 
-def knn_kernel(Xq, ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandwidth=None,
-               bandwidth_scale=1.0, S=None, impl=None):
-    """Raw (unsymmetrised) kNN / alpha-decay kernel from the rows of ``Xq`` to ``ref`` as DeviceCSR.
+class TcFlavour(NamedTuple):
+    """One tensor-core search flavour (csrc/search_tc.cu).  Its operand rows are whole 32-byte k-steps (SWIZZLE_128B
+    blocks plus SWIZZLE_32B tail blocks) holding the d centred features, the |y|^2 column and ``spare`` more.
+    (Padding bf16 rows to whole 128-byte blocks was measured slower: 699 vs 682 ms at d = 100 -- the extra MMAs cost
+    more than the tail blocks.)"""
+    name: str
+    dtype: int          # dtype code of the C ABI
+    step: int           # elements per k-step: 8 tf32, 16 bf16 / fp16
+    spare: int          # float16 operands keep one more column: the low part of |y|^2
+    max_steps: int      # k-steps of the resident query tile (the fp16x2 flavour streams longer rows in chunks)
+    list_cap: int       # candidates per row: 2 lists x 32, one list of 64 for the one-product flavour
+    eps_rel: object     # relative bound of its squared distances (certification)
+    fp16: bool          # operands are the data scaled by fp16_scale, in float16
+    operand: int        # dtype code of the operands it reads and of its radius pass
+
+    def kp(self, d):
+        return (d + 1 + self.spare + self.step - 1) // self.step * self.step
+
+    def fits(self, d):
+        return self.kp(d) // self.step <= self.max_steps
+
+
+TC_FLAVOURS = (                                               # indexed by dtype code
+    TcFlavour("tc", 0, 8, 0, 13, 32, eps_rel_tc, False, 0),           # 3xTF32
+    TcFlavour("tc16", 1, 16, 0, 8, 32, eps_rel_tc16, False, 1),       # bf16x3
+    TcFlavour("tch", 2, 16, 1, 32, 32, eps_rel_tch, True, 2),         # fp16x2: two products
+    TcFlavour("tch1", 3, 16, 1, 8, 64, eps_rel_tch1, True, 2),        # fp16, one product: reads the fp16x2 operands
+)
+FLAVOURS = {f.name: f for f in TC_FLAVOURS}
+# GTB_SEARCH_IMPL is a preference: a flavour that cannot take the shape (feature count beyond the resident query tile,
+# knn beyond the candidate lists) hands over to the next one
+FALLBACK = {"auto": (AUTO_TC, "tch", "tc16", "tc", "simt"), "tc": ("tc", "tc16", "simt"), "tc16": ("tc16", "tc", "simt"),
+            "tch": ("tch", "tc16", "tc", "simt"), "tch1": ("tch1", "tch", "tc16", "tc", "simt"), "simt": ("simt",)}
+TC_CLUSTER = 2           # CTAs per cluster sharing each reference tile by TMA multicast
+SEED_STRIDE = 16         # the seed sweep of the one-product flavour visits every 16th reference tile
+SearchPlan = namedtuple("SearchPlan", "impl ls qtiles S ntau seeded")
+
+
+def plan_search(want, d, n_pad, metric, knn, kmax, binary):
+    """Flavour and list shapes of a kNN search: ``want`` = GTB_SEARCH_IMPL, ``d`` features, ``n_pad`` padded
+    reference rows, ``knn`` / ``kmax`` (0 = none) neighbours per row, ``binary`` = no decay.  Returns a SearchPlan:
+    the flavour (a key of FLAVOURS, or "simt"), entries per candidate list ``ls`` and query tiles per CTA ``qtiles``
+    (tensor cores; None for simt), candidates per row ``S``, thresholds per row ``ntau``, and whether a seed sweep
+    sets the starting thresholds."""
+    # a strided sample needs enough tiles to carry the order statistic: 32 sampled tiles at least
+    seedable = n_pad // 128 >= 32 * SEED_STRIDE
+    if metric == "cityblock":
+        impl = "simt"                                     # |x - y| has no GEMM form: CUDA-core L1 kernel only
+    elif want not in FALLBACK:
+        raise ValueError("GTB_SEARCH_IMPL must be auto, tc, tc16, tch, tch1 or simt (got %r)" % (want,))
+    else:
+        # auto: the one-product flavour pays off only with seeded thresholds (cold, its list of 64 costs more than the
+        # second product saves: C3 at 50k x 50 6.7 ms against 2.5 ms) -- unless the longer list is what knn needs
+        impl = next(c for c in FALLBACK[want] if c == "simt" or (
+            FLAVOURS[c].fits(d) and knn + 8 <= FLAVOURS[c].list_cap
+            and not (c == "tch1" and want == "auto" and not seedable and knn + 8 <= 32)))
+    if impl == "simt":
+        S = choose_S(knn, binary)
+        return SearchPlan(impl, None, None, S, 1, False)
+    f = FLAVOURS[impl]
+    if f.dtype == 3:
+        ls, qtiles = 32, 2                                # one product: one list of 64 per row, always two tiles
+    else:
+        # short lists (16) halve the selection work of the sweep when the neighbourhood asked for is small -- rows
+        # whose kernel support is wider fail certification and are finished by the radius pass.  The fp16x2 flavour
+        # with rows of 8 k-steps runs two query tiles per CTA and keeps ONE list of 32 per row.  knn_max neighbours
+        # must fit the lists as well.
+        two_tiles = f.dtype == 2 and f.kp(d) <= 128
+        ls = 16 if max(knn, kmax) + 8 <= (32 if two_tiles else 16) else 32
+        qtiles = 2 if two_tiles and ls == 16 else 1
+    return SearchPlan(impl, ls, qtiles, 2 * ls, 2, f.dtype == 3 and seedable)
+
+
+def _sweep_tc(plan, qry, ref):
+    """Tensor-core sweep: (candidates, tau, query norms, eps_rel, fp16 scale)."""
+    f = FLAVOURS[plan.impl]
+    nq = qry.n
+    # grid-wide pacing of the TMA producers: one caller-owned device word per launch (no library state)
+    pace = _empty((1,), torch.int32)
+    scale = fp16_scale(max(qry.norm_max(), ref.norm_max())) if f.fp16 else 1.0
+    q_hi, q_lo, q_n2 = qry.tc(0, f.dtype, scale)
+    r_hi, r_lo, _ = ref.tc(1, f.dtype, scale)
+    Kp = ref.kp(f.dtype)
+    cand = _empty((nq, plan.S), torch.int32)
+    tau = _empty((nq, plan.ntau), torch.float32)
+    scratch = _empty((E.lib().gtb_tc_scratch_bytes(qry.n_pad),), torch.uint8)
+    s2 = scale * scale
+    qn2_s = q_n2 * s2 if f.fp16 else q_n2
+    if f.dtype == 3:
+        seed = None
+        if plan.seeded:
+            # threshold seeds: the 8th smallest tile minimum over every stride-th reference tile (6 % of the tensor
+            # work of a sweep, no selection work); it sits near the (8 stride)-th smallest distance overall, so the
+            # full sweep starts with a threshold that admits ~8 stride points per row instead of climbing down from
+            # +inf (64 ln(N / 64) threshold updates)
+            seed = _empty((nq, plan.ntau), torch.float32)
+            E.call("gtb_knn_seed_tc", q_hi, qn2_s, nq, qry.n_pad, r_hi, ref.n, ref.n_pad, Kp, TC_CLUSTER, SEED_STRIDE,
+                   seed, pace)
+        E.call("gtb_knn_topk_tc_seeded", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, ref.n, ref.n_pad, Kp, f.dtype,
+               plan.ls, TC_CLUSTER, plan.qtiles, seed, 1, cand, scratch, tau, pace)
+    else:
+        E.call("gtb_knn_topk_tc", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, ref.n, ref.n_pad, Kp, f.dtype, plan.ls,
+               TC_CLUSTER, plan.qtiles, cand, scratch, tau, pace)
+    if f.fp16:
+        tau = tau / s2                                   # scaled squared distances -> data units (inf stays inf)
+    return cand, tau, q_n2, f.eps_rel(ref.d), scale
+
+
+def _sweep_simt(plan, qry, ref):
+    """CUDA-core sweep: (candidates, tau, query norms, eps_rel, 1.0)."""
+    nq = qry.n
+    tau = _empty((nq,), torch.float32)
+    cand = _empty((nq, plan.S), torch.int32)
+    if ref.metric == "cityblock":
+        q_n2 = qry.l1_norms()[0] if ref.is64 else None       # float32 inputs: the search copy is exact
+        E.call("gtb_knn_topk_simt_l1", qry.XT, nq, qry.n_pad, ref.XT, ref.n, ref.n_pad, ref.d_pad, plan.S, cand, tau)
+        return cand, tau, q_n2, eps_rel_l1(ref.d), 1.0
+    E.call("gtb_knn_topk_simt", qry.XT, qry.n2, nq, qry.n_pad, ref.XT, ref.n2, ref.n, ref.n_pad, ref.d_pad, plan.S,
+           cand, tau)
+    return cand, tau, qry.n2, eps_rel_simt(ref.d), 1.0
+
+
+def _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out, nzero, x64, kern):
+    """Rows the refine could not certify: every reference point inside the row's radius ``lim2``, refined in float64
+    and merged into ``n_keep`` / ``bw_out`` / ``nzero``.  Returns the rows' segments (ptr, idx, val, n_keep)."""
+    nr, d = ref.n, ref.d
+    nt = todo_rows.shape[0]
+    nt_pad = (nt + 127) // 128 * 128
+    lim_t = _zeros((nt_pad,), torch.float32)
+    lim_t[:nt] = lim2[todo_rows.long()]
+    f = FLAVOURS.get(plan.impl)
+    if f:
+        # the radius rows form their own (small) query operand; build it from the gathered rows
+        sub = SearchOperand(qry.X[todo_rows.long()].contiguous(), mean=ref.mean, metric=ref.metric)
+        s_hi, s_lo, s_n2 = sub.tc(0, f.dtype, scale)
+        r_hi, r_lo, _ = ref.tc(1, f.dtype, scale)
+        if f.fp16:
+            s_n2 = s_n2 * (scale * scale)
+            lim_t = lim_t * (scale * scale)
+        pace = _empty((1,), torch.int32)
+    else:
+        QT = _empty((ref.d_pad, nt_pad), torch.float32)
+        qn2 = _empty((nt_pad,), torch.float32)
+        E.call("gtb_gather_operand", qry.XT, qry.n_pad, qry.n2, todo_rows, nt, QT, nt_pad, ref.d_pad, qn2)
+    capacity = max(1 << 20, nt * 4 * plan.S)
+    while True:
+        pairs = _empty((capacity, 2), torch.int32)
+        counter = _zeros((1,), torch.int64)
+        rowcnt = _zeros((nt_pad,), torch.int32)
+        if f:
+            # (the one-product flavour hands its uncertified rows to the two-product sweep on the same operands)
+            E.call("gtb_knn_radius_tc", s_hi, s_lo, s_n2, lim_t, nt, nt_pad, r_hi, r_lo, nr, ref.n_pad, ref.kp(f.dtype),
+                   f.operand, TC_CLUSTER, pairs, capacity, counter, rowcnt, pace)
+        elif ref.metric == "cityblock":
+            E.call("gtb_knn_radius_simt_l1", QT, lim_t, nt, nt_pad, ref.XT, nr, ref.n_pad, ref.d_pad, pairs,
+                   capacity, counter, rowcnt)
+        else:
+            E.call("gtb_knn_radius_simt", QT, qn2, lim_t, nt, nt_pad, ref.XT, ref.n2, nr, ref.n_pad, ref.d_pad,
+                   pairs, capacity, counter, rowcnt)
+        npairs = int(counter.item())
+        if npairs <= capacity:
+            break
+        capacity = npairs
+    _STATS.update(radius_pairs=npairs)
+    seg_ptr = exclusive_scan(rowcnt[:nt].contiguous())
+    seg_idx = _empty((max(npairs, 1),), torch.int32)
+    seg_val = _empty((max(npairs, 1),), torch.float64)
+    cursor = _empty((nt,), torch.int32)
+    E.call("gtb_scatter_pairs", pairs, npairs, seg_ptr, cursor, nt, seg_idx)
+    n_keep_t = _empty((nt,), torch.int32)
+    overflow = _empty((1,), torch.int32)
+    longest = int(rowcnt.max().item())
+    cap = 64
+    while cap < longest:
+        cap *= 2
+    if cap > BALL_CAP:
+        raise RowTooLong(
+            "a row has {} neighbours inside the kernel radius; the sparse kNN pipeline handles rows of up to {} "
+            "(a kernel this dense calls for graphtype='exact', which evaluates every pair)".format(longest, BALL_CAP))
+    E.call("gtb_refine_ball", qry.X, todo_rows, status, nt, ref.X, d, x64, seg_ptr, seg_idx, seg_val, *kern, n_keep_t,
+           n_keep, bw_out, nzero, overflow, cap)
+    return seg_ptr, seg_idx, seg_val, n_keep_t
+
+
+def knn_kernel(ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandwidth=None, bandwidth_scale=1.0):
+    """Raw (unsymmetrised) kNN / alpha-decay kernel from the rows of ``qry`` (default ``ref``) to ``ref`` as DeviceCSR.
 
     Semantics = reference ``kNNGraph.build_kernel_to_data`` (graphs.py:819-982) with the float64
     path: ``knn`` is the effective neighbour count (callers pass knn+1 for the self-including
@@ -509,133 +656,36 @@ def knn_kernel(Xq, ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, b
     info['nzero'] (zero-distance candidates per row, for duplicate warnings).
     """
     E.require_cuda()
-    if qry is None:
-        qry = ref
+    qry = ref if qry is None else qry
     nq, nr, d = qry.n, ref.n, ref.d
     if qry.is64 != ref.is64 or qry.metric != ref.metric:
         raise ValueError("query and reference operands must have the same dtype and metric")
     x64 = int(ref.is64) | (METRIC_CODE[ref.metric] << 1)            # x_kind of the refine entry points
-    l1 = ref.metric == "cityblock"
     binary = decay is None
     knn = int(min(knn, nr))
     kmax = 0 if knn_max is None else int(knn_max)
     if kmax >= nr:
         kmax = 0
-    if l1:
-        impl = "simt"
-    if impl is None:
-        # GTB_SEARCH_IMPL is a preference: a flavour that cannot take this shape (feature count beyond the
-        # resident query tile, knn beyond the 2 x 32 candidate lists) hands over to the next one
-        want = default_impl()
-        order = {"auto": (AUTO_TC,) + tuple(x for x in ("tch", "tc16", "tc") if x != AUTO_TC) + ("simt",),
-                 "tc": ("tc", "tc16", "simt"), "tc16": ("tc16", "tc", "simt"), "tch": ("tch", "tc16", "tc", "simt"),
-                 "tch1": ("tch1", "tch", "tc16", "tc", "simt"), "simt": ("simt",)}.get(want)
-        if order is None:
-            raise ValueError("GTB_SEARCH_IMPL must be auto, tc, tc16, tch, tch1 or simt (got %r)" % (want,))
-        impl = "simt"
-        for cand_impl in order:
-            # auto: the one-product flavour pays off only with seeded thresholds, i.e. when the reference set is
-            # large enough for a strided sample (cold, its list of 64 costs more than the second product saves:
-            # C3 at 50k x 50 6.7 ms against 2.5 ms) -- unless the longer list is what the request needs
-            if (cand_impl == "tch1" and want == "auto" and not seedable(ref) and knn + 8 <= 32):
-                continue
-            # neighbours asked for must fit the candidate lists: 2 x 32 entries, one list of 64 for tch1
-            if cand_impl == "simt" or (knn + 8 <= (64 if cand_impl == "tch1" else 32) and S in (None, 32, 64)
-                                       and ref.tc_ok(TC_DTYPE[cand_impl])):
-                impl = cand_impl
-                break
-    dev = _dev()
-    ntau = 1
-    tcd = TC_DTYPE.get(impl, 0)
-    tc_scale = 1.0
-    if impl in TC_DTYPE:
-        if not ref.tc_ok(tcd):
-            raise ValueError("tensor-core search: d = {} does not fit the resident query tile".format(d))
-        import os
-        # two candidate lists per row (one per epilogue group) of `ls` entries each.  Short lists (16) halve the
-        # selection work of the sweep; they are used when the neighbourhood asked for is small (knn + 8 <= 16) --
-        # rows whose kernel support is wider fail certification and are finished by the radius pass.
-        want = max(knn, kmax)                                   # knn_max neighbours must fit the lists as well
-        # (fp16x2 runs two query tiles per CTA and keeps ONE list of 32 per row, which covers want + 8 <= 32)
-        two_tiles = tcd == 2 and int(os.environ.get("GTB_TC_QTILES", "2")) == 2 and ref.kp(2) <= 128
-        short_ok = want + 8 <= (32 if two_tiles else 16)
-        ls = int(os.environ.get("GTB_TC_LIST", "16" if short_ok else "32"))
-        qtiles = 2 if (two_tiles and ls == 16) else 1
-        if tcd == 3:
-            ls, qtiles = 32, 2                                  # one product: one list of 64 per row, always two tiles
-        if ls not in (16, 32) or knn > ls * qtiles:
-            raise ValueError("GTB_TC_LIST must be 16 or 32 and >= knn")
-        S, stride, ntau = 2 * ls, 2 * ls, 2
-        cluster = min(tc_cluster(), 2) if tcd else tc_cluster()
-        if cluster not in (1, 2, 4):
-            raise ValueError("GTB_TC_CLUSTER must be 1, 2 or 4")
-        # grid-wide pacing of the TMA producers: one caller-owned device word per launch (no library state)
-        pace = _empty((1,), torch.int32) if int(os.environ.get("GTB_TC_PACING", "1")) else None
-        if knn > (64 if tcd == 3 else 32):
-            raise NotImplementedError("knn={} exceeds the tensor-core candidate lists (2 x 32)".format(knn))
-        eps_rel = (eps_rel_tc, eps_rel_tc16, eps_rel_tch, eps_rel_tch1)[tcd](d)
-        if tcd >= 2:
-            tc_scale = fp16_scale(max(qry.norm_max(), ref.norm_max()))
-        q_hi, q_lo, q_n2 = qry.tc(0, tcd, tc_scale)
-        r_hi, r_lo, _ = ref.tc(1, tcd, tc_scale)
-        Kp = ref.kp(tcd)
-        cand = _empty((nq, stride), torch.int32)
-        tau = _empty((nq, ntau), torch.float32)
-        scratch = _empty((E.lib().gtb_tc_scratch_bytes(qry.n_pad),), torch.uint8)
-        s2 = tc_scale * tc_scale
-        # qtiles == 2: two query tiles per CTA share every reference stage (half the L2 traffic per MMA)
-        qn2_s = q_n2 * s2 if tcd >= 2 else q_n2
-        seed = None
-        stride_s = seed_stride()
-        if tcd == 3 and seedable(ref):
-            # threshold seeds: the 8th smallest tile minimum over every stride-th reference tile (6 % of the tensor work
-            # of a sweep, no selection work); it sits near the (8 stride)-th smallest distance overall, so the full
-            # sweep starts with a threshold that admits ~8 stride points per row instead of climbing down from +inf
-            # (64 ln(N / 64) threshold updates)
-            seed = _empty((nq, ntau), torch.float32)
-            E.call("gtb_knn_seed_tc", q_hi, qn2_s, nq, qry.n_pad, r_hi, nr, ref.n_pad, Kp, cluster, stride_s, seed, pace)
-        if tcd == 3:
-            E.call("gtb_knn_topk_tc_seeded", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, nr, ref.n_pad, Kp, tcd, ls,
-                   cluster, qtiles, seed, 1, cand, scratch, tau, pace)
-        else:
-            E.call("gtb_knn_topk_tc", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, nr, ref.n_pad, Kp, tcd, ls,
-                   cluster, qtiles, cand, scratch, tau, pace)
-        del seed
-        if tcd >= 2:
-            tau = tau / s2                                   # scaled squared distances -> data units (inf stays inf)
-        del scratch
-    elif impl == "simt":
-        if S is None:
-            S = choose_S(knn, binary)
-        stride = S
-        tau = _empty((nq,), torch.float32)
-        cand = _empty((nq, S), torch.int32)
-        if l1:
-            eps_rel = eps_rel_l1(d)
-            q_n2 = qry.l1_norms()[0] if ref.is64 else None       # float32 inputs: the search copy is exact
-            E.call("gtb_knn_topk_simt_l1", qry.XT, nq, qry.n_pad, ref.XT, nr, ref.n_pad, ref.d_pad, S, cand, tau)
-        else:
-            eps_rel = eps_rel_simt(d)
-            q_n2 = qry.n2
-            E.call("gtb_knn_topk_simt", qry.XT, qry.n2, nq, qry.n_pad, ref.XT, ref.n2, nr, ref.n_pad, ref.d_pad, S,
-                   cand, tau)
-    else:
-        raise ValueError("unknown impl %r" % (impl,))
+    plan = plan_search(default_impl(), d, ref.n_pad, ref.metric, knn, kmax, binary)
+    sweep = _sweep_simt if plan.impl == "simt" else _sweep_tc
+    cand, tau, q_n2, eps_rel, scale = sweep(plan, qry, ref)
 
     # bandwidth argument
     bw_mode, bw_fixed = 0, None
     if not binary and bandwidth is not None:
         if np.ndim(bandwidth) == 0:
-            bw_mode, bw_fixed = 1, torch.tensor([float(bandwidth)], dtype=torch.float64, device=dev)
+            bw_mode, bw_fixed = 1, torch.tensor([float(bandwidth)], dtype=torch.float64, device=_dev())
         else:
             bw_arr = np.asarray(bandwidth, dtype=np.float64).reshape(-1)
             if bw_arr.shape[0] != nq:
                 raise ValueError("bandwidth must be a scalar or have one entry per row ({}), got {}".format(
                     nq, bw_arr.shape[0]))
-            bw_mode, bw_fixed = 2, torch.from_numpy(bw_arr).to(dev)
-    decay_f = -1.0 if binary else float(decay)
-    thresh_f = 1.0 if binary else float(thresh)
+            bw_mode, bw_fixed = 2, torch.from_numpy(bw_arr).to(_dev())
+    # kernel parameters, in the order both refine entry points take them
+    kern = (knn, kmax, -1.0 if binary else float(decay), 1.0 if binary else float(thresh), bw_fixed, bw_mode,
+            float(bandwidth_scale))
 
+    S = plan.S
     st_idx = _empty((nq, S), torch.int32)
     st_val = _empty((nq, S), torch.float64)
     n_keep = _empty((nq,), torch.int32)
@@ -643,80 +693,27 @@ def knn_kernel(Xq, ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, b
     lim2 = _empty((nq,), torch.float32)
     status = _empty((nq,), torch.int32)
     nzero = _empty((nq,), torch.int32)
-    maxnorm = (ref.l1_norms()[1] if ref.is64 else 0.0) if l1 else ref.maxnorm
-    E.call("gtb_refine_topk", qry.X, nq, ref.X, d, x64, cand, S, stride, tau, ntau, q_n2, maxnorm, eps_rel, knn, kmax, decay_f,
-           thresh_f, bw_fixed, bw_mode, float(bandwidth_scale), st_idx, st_val, n_keep, bw_out, lim2, status, nzero)
+    maxnorm = (ref.l1_norms()[1] if ref.is64 else 0.0) if ref.metric == "cityblock" else ref.maxnorm
+    E.call("gtb_refine_topk", qry.X, nq, ref.X, d, x64, cand, S, S, tau, plan.ntau, q_n2, maxnorm, eps_rel, *kern,
+           st_idx, st_val, n_keep, bw_out, lim2, status, nzero)
 
     todo_rows = _empty((nq,), torch.int32)
     count = _empty((1,), torch.int32)
     E.call("gtb_compact_todo", status, nq, todo_rows, count)
     nt = int(count.item())                       # host sync #1
-    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=impl, euclidean_fallback_rows=0)
+    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=plan.impl, euclidean_fallback_rows=0)
 
-    seg_ptr = seg_idx = seg_val = n_keep_t = None
+    seg = (None,) * 4
     if nt > 0:
         todo_rows = todo_rows[:nt].contiguous()
-        nt_pad = (nt + 127) // 128 * 128
-        lim_t = torch.zeros((nt_pad,), dtype=torch.float32, device=dev)
-        lim_t[:nt] = lim2[todo_rows.long()]
-        if impl in TC_DTYPE:
-            # the radius rows form their own (small) query operand; build it from the gathered rows
-            sub = SearchOperand(qry.X[todo_rows.long()].contiguous(), mean=ref.mean, metric=ref.metric)
-            s_hi, s_lo, s_n2 = sub.tc(0, tcd, tc_scale)
-            r_hi, r_lo, _ = ref.tc(1, tcd, tc_scale)
-            if tcd >= 2:
-                s_n2 = s_n2 * (tc_scale * tc_scale)
-                lim_t = lim_t * (tc_scale * tc_scale)
-        else:
-            QT = _empty((ref.d_pad, nt_pad), torch.float32)
-            qn2 = _empty((nt_pad,), torch.float32)
-            E.call("gtb_gather_operand", qry.XT, qry.n_pad, qry.n2, todo_rows, nt, QT, nt_pad, ref.d_pad, qn2)
-        capacity = max(1 << 20, nt * 4 * S)
-        while True:
-            pairs = _empty((capacity, 2), torch.int32)
-            counter = _zeros((1,), torch.int64)
-            rowcnt = _zeros((nt_pad,), torch.int32)
-            if impl in TC_DTYPE:
-                # (the one-product flavour hands its uncertified rows to the two-product sweep on the same operands)
-                E.call("gtb_knn_radius_tc", s_hi, s_lo, s_n2, lim_t, nt, nt_pad, r_hi, r_lo, nr, ref.n_pad, Kp,
-                       min(tcd, 2), cluster, pairs, capacity, counter, rowcnt, pace)
-            elif l1:
-                E.call("gtb_knn_radius_simt_l1", QT, lim_t, nt, nt_pad, ref.XT, nr, ref.n_pad, ref.d_pad, pairs,
-                       capacity, counter, rowcnt)
-            else:
-                E.call("gtb_knn_radius_simt", QT, qn2, lim_t, nt, nt_pad, ref.XT, ref.n2, nr, ref.n_pad, ref.d_pad,
-                       pairs, capacity, counter, rowcnt)
-            npairs = int(counter.item())
-            if npairs <= capacity:
-                break
-            capacity = npairs
-        _STATS.update(radius_pairs=npairs)
-        seg_ptr = exclusive_scan(rowcnt[:nt].contiguous())
-        seg_idx = _empty((max(npairs, 1),), torch.int32)
-        seg_val = _empty((max(npairs, 1),), torch.float64)
-        cursor = _empty((nt,), torch.int32)
-        E.call("gtb_scatter_pairs", pairs, npairs, seg_ptr, cursor, nt, seg_idx)
-        n_keep_t = _empty((nt,), torch.int32)
-        overflow = _empty((1,), torch.int32)
-        longest = int(rowcnt.max().item())
-        cap = 64
-        while cap < longest:
-            cap *= 2
-        if cap > BALL_CAP:
-            raise RowTooLong(
-                "a row has {} neighbours inside the kernel radius; the sparse kNN pipeline handles rows of up to {} "
-                "(a kernel this dense calls for graphtype='exact', which evaluates every pair)".format(
-                    longest, BALL_CAP))
-        E.call("gtb_refine_ball", qry.X, todo_rows, status, nt, ref.X, d, x64, seg_ptr, seg_idx, seg_val, knn, kmax,
-               decay_f, thresh_f, bw_fixed, bw_mode, float(bandwidth_scale), n_keep_t, n_keep, bw_out, nzero,
-               overflow, cap)
+        seg = _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out, nzero, x64, kern)
 
     indptr = exclusive_scan(n_keep)
     nnz = int(indptr[-1].item())                 # host sync #2
     out_idx = _empty((nnz,), torch.int32)
     out_val = _empty((nnz,), torch.float64)
-    E.call("gtb_csr_gather", st_idx, st_val, n_keep, status, indptr, nq, S, todo_rows if nt else None, nt,
-           seg_ptr, seg_idx, seg_val, n_keep_t, out_idx, out_val)
+    E.call("gtb_csr_gather", st_idx, st_val, n_keep, status, indptr, nq, S, todo_rows if nt else None, nt, *seg,
+           out_idx, out_val)
     _STATS.update(nnz_raw=nnz)
     csr = DeviceCSR(indptr, out_idx, out_val, (nq, nr))
     return csr, {"bandwidth": bw_out, "nzero": nzero}

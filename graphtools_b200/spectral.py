@@ -157,7 +157,7 @@ def assign_nearest(X, centers):
     exact float64 re-evaluation -- and the squared distance to it."""
     ref = pipeline.SearchOperand(centers.contiguous())
     qry = pipeline.SearchOperand(X, mean=ref.mean)
-    nearest, _ = pipeline.knn_kernel(None, ref, qry, knn=1, decay=None)
+    nearest, _ = pipeline.knn_kernel(ref, qry, knn=1, decay=None)
     labels = nearest.indices.to(torch.int64)
     d2 = ((X - centers[labels]) ** 2).sum(dim=1)
     return labels, d2

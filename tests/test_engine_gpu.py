@@ -421,15 +421,17 @@ def test_symmetrize_normalize_matches_scipy(mode, theta, n, density, hub):
     assert flags == 2
 
 
-@pytest.mark.parametrize("mode,theta", [("+", None), ("*", None), ("mnn", 0.3)])
+@pytest.mark.parametrize("mode,theta", [("+", None), ("*", None), ("mnn", 0.0), ("mnn", 0.3), ("mnn", 0.5),
+                                        ("mnn", 1.0)])
 def test_sharded_symmetrise_merge_matches_global(mode, theta):
     """The multi-GPU path on one device: the rows of two shards are bucketed by route_count / route_fill, the
     records a rank would receive are turned into the transposed rows (records_count / scatter / sort) and merged --
-    bit-identical to the single-GPU symmetrise + normalise."""
+    bit-identical to the single-GPU symmetrise + normalise.  MNN weights from theta = 0 (the larger of the two
+    directions) to theta = 1 (the smaller: one-way edges drop out of the merged rows)."""
     from graphtools_b200 import distributed as gd
     X, _ = synth.gaussian_mixture(3000, 20, n_clusters=4, intrinsic_dim=5, seed=9)
     ref = pipeline.SearchOperand(_dev(X))
-    R, _ = pipeline.knn_kernel(None, ref, ref, knn=6, decay=10, thresh=1e-3)
+    R, _ = pipeline.knn_kernel(ref, ref, knn=6, decay=10, thresh=1e-3)
     K, P, deg, _ = pipeline.symmetrize_normalize(R, mode, theta, 0.0)
     Kh, Ph = K.to_scipy(), K.to_scipy(P)
     Rh = R.to_scipy()
