@@ -35,8 +35,14 @@ _SIGS = {
     "gtb_knn_topk_tc": ([_P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, c_int, c_int, _P,
                          _P, _P, _P, _P], 1),
     "gtb_knn_topk_tc_seeded": ([_P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, c_int, c_int,
-                                _P, c_int, _P, _P, _P, _P, _P], 1),
+                                _P, c_int, _P, _P, _P, _P, _P, _P, _P, _P], 1),
     "gtb_knn_seed_tc": ([_P, _P, c_int64, c_int64, _P, c_int64, c_int64, c_int, c_int, c_int, _P, _P, _P], 1),
+    "gtb_order_assign": ([_P, c_int64, c_int, c_int, _P, _P], 1),
+    "gtb_order_sort": ([_P, c_int64, c_int, _P, _P, _P], 3),
+    "gtb_tile_geometry": ([_P, c_int64, c_int, c_int, _P, c_int64, c_int64, _P, _P, _P], 1),
+    "gtb_tile_lists_count": ([_P, _P, _P, c_int64, _P, _P, c_int64, c_int, _P, _P, _P], 1),
+    "gtb_tile_lists_fill": ([_P, c_int64, c_int64, _P, _P, _P], 1),
+    "gtb_unpermute_candidates": ([_P, _P, c_int64, c_int, c_int, _P, _P, _P, _P, _P], 1),
     "gtb_knn_radius_tc": ([_P, _P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, _P, c_int64,
                            _P, _P, _P, _P], 1),
     "gtb_refine_topk": ([_P, c_int64, _P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_float, c_double, c_int, c_int64, c_double,
@@ -86,6 +92,8 @@ _SIGS = {
     "gtb_sp_store_rows": ([_P, c_int, c_int64, _P, c_int, _P, c_int64, _P], 1),
     "gtb_sp_finish": ([_P, c_int64, _P], 1),
 }
+# entry points whose last pointer arguments are optional: a call may omit them (NULL)
+_OPTIONAL_TAIL = {"gtb_knn_topk_tc_seeded": 3}
 _PLAIN = {
     "gtb_last_error": ([], ctypes.c_char_p),
     "gtb_version": ([], c_int),
@@ -98,6 +106,7 @@ _PLAIN = {
     "gtb_tc_scratch_bytes": ([c_int64], c_int64),
     "gtb_gemm_max_k": ([], c_int),
     "gtb_knn_seed_k": ([], c_int),
+    "gtb_order_ws_elems": ([c_int64, c_int], c_int64),
     "gtb_sp_ws_bytes": ([c_int64, c_int], c_int64),
 }
 
@@ -171,6 +180,8 @@ def call(name, *args):
     conv = []
     for a, t in zip(args, argtypes):
         conv.append(_ptr(a) if t is _P else a)
+    if 0 < len(argtypes) - 1 - len(conv) <= _OPTIONAL_TAIL.get(name, 0):
+        conv += [None] * (len(argtypes) - 1 - len(conv))
     assert len(conv) == len(argtypes) - 1, (name, len(conv), len(argtypes))
     timed = timing is not None and (timing_only is None or key in timing_only)
     if timed:

@@ -13,4 +13,4 @@ void gtb_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* gtb_last_error(void) { return g_err; }
-extern "C" int gtb_version(void) { return 202; }   // + sqeuclidean and correlation metrics (x_kind bits 1-3, dense metric 3)
+extern "C" int gtb_version(void) { return 203; }   // + tile lists of gtb_knn_topk_tc_seeded, locality order (csrc/order.cu)

@@ -83,6 +83,10 @@ struct TcParams {
   // and merge_pieces_kernel builds the rows.  split_k = 0: ordinary launch.  q_unit0: first cluster-unit of the launch.
   int64_t q_unit0, split_k, split_row0, split_rows;
   uint2* piece_buf; uint2* piece_meta;
+  // TOPK, listed (gtb_knn_topk_tc_seeded with tile lists): unit u = the CL x QT query tiles one cluster sweeps in a round,
+  // rows [u * CL * QT * 128, ...); it visits the reference tiles unit_tiles[unit_ptr[u] .. unit_ptr[u + 1]) only.  Round r
+  // of cluster c takes slot r * n_clusters + c (c mirrored in odd rounds) of unit_order, longest list first.
+  const int64_t* unit_ptr; const int32_t* unit_tiles; const int32_t* unit_order; int64_t n_units;
   const float* qn2;
   int32_t* cand_idx; uint2* cand_buf; float* tau;          // TOPK: out [nq][2*TC_S], scratch [nq_pad][2][TC_CAP], tau [nq][2]
   const float* lim2; int2* pairs; unsigned long long capacity; unsigned long long* counter; int32_t* rowcnt;
@@ -232,10 +236,13 @@ __device__ __forceinline__ void tc_commit_mc_pred(uint32_t bar, uint16_t mask, u
 // drops to two products: 57 KB per stage and SM = 1340 clk against 896 clk of MMAs.)
 // PIECE: the second launch of a split top-k sweep (own instantiation: the ordinary sweep sits exactly at the register
 // budget ptxas grants this kernel, and one more live value in its epilogue costs 13 % of the sweep)
+// LISTED: the pruned one-product top-k sweep -- every unit sweeps its own list of reference tiles (TcParams::unit_ptr);
+// no grid-wide pacing (the units do not stream the same tiles) and no split last round
 // WIDE: operand rows longer than 8 k-steps (129 .. 512 float16 elements, i.e. d up to 510): the query tile still
 // lives in TMEM (hi parts only: 8 columns per k-step, up to 256 columns beside two accumulators), the reference tiles
 // stream in CHUNKS of 8 k-steps -- a stage is one (tile, chunk) pair and the accumulator collects all chunks of a tile.
-template <int MODE, int CL, int FMT, int LS, int QT, bool PIECE = false, bool WIDE = false>  // MODE 0 = TOPK, 1 = RADIUS, 2 = SEED
+template <int MODE, int CL, int FMT, int LS, int QT, bool PIECE = false, bool WIDE = false,   // MODE 0 = TOPK, 1 = RADIUS,
+          bool LISTED = false>                                                                   // 2 = SEED
 __global__ void __launch_bounds__(TC_THREADS, 1)
 search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant__ CUtensorMap mBht,
                  const __grid_constant__ CUtensorMap mBl, const __grid_constant__ CUtensorMap mBlt,
@@ -254,6 +261,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
   static_assert(MODE != 2 || (FMT == 3 && QT == 2), "seed sweeps use the one-product flavour");
   static_assert(FMT != 3 || QT == 2, "the one-product flavour runs two query tiles per CTA");
   static_assert(!WIDE || (FMT == 2 && QT == 1 && !PIECE), "wide operand rows: fp16x2, one query tile per CTA");
+  static_assert(!LISTED || (MODE == 0 && FMT == 3 && !PIECE && !WIDE), "tile lists: one-product top-k sweep");
   constexpr int LSO = (QT == 2) ? 2 * LS : LS;               // entries of one output list
   // candidate buffer of one list: a row owns TC_GROUPS * TC_CAP slots of scratch; the single long list of QT == 2 may
   // use all of them (fewer compactions between the seeded threshold and the final selection)
@@ -299,9 +307,17 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
   const int64_t tstride = (MODE != 1) ? p.tile_stride : 1;
   const int64_t tiles_left = (p.nr_pad / TC_N + tstride - 1) / tstride - tile0;
   const int64_t ntiles = tiles_left < p.tiles_per_split ? tiles_left : p.tiles_per_split;
+  // LISTED: the unit of a round (slots past the last unit are padding units: rows beyond nq_pad, no tiles) and its list
+  auto unit_of = [&](int64_t round) -> int64_t {
+    const int64_t slot = round * n_clusters + ((round & 1) ? (n_clusters - 1 - qcluster) : qcluster);
+    return slot < p.n_units ? (int64_t)p.unit_order[slot] : slot;
+  };
+  auto list_lo = [&](int64_t u) -> int64_t { return u < p.n_units ? p.unit_ptr[u] : 0; };
+  auto list_len = [&](int64_t u) -> int64_t { return u < p.n_units ? p.unit_ptr[u + 1] - p.unit_ptr[u] : 0; };
   // first query row of (round, query tile qt of this CTA)
   auto q0_of = [&](int64_t round, int qt) {
-    return ((((PIECE ? p.q_unit0 : 0) + qcluster + round * n_clusters) * CL + (blockIdx.x % CL)) * QT + qt) * TC_M;
+    const int64_t u = LISTED ? unit_of(round) : (PIECE ? p.q_unit0 : 0) + qcluster + round * n_clusters;
+    return ((u * CL + (blockIdx.x % CL)) * QT + qt) * TC_M;
   };
   static_assert(!PIECE || (MODE == 0 && FMT == 3), "piece launches belong to the one-product top-k sweep");
   auto btile = [&](int64_t round, int64_t t) { return (tile0 + ((round & 1) ? (ntiles - 1 - t) : t)) * tstride; };
@@ -442,7 +458,9 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
     if (lane == 0) {
       int64_t it = 0;                              // running stage counter across rounds
       for (int64_t round = 0; round < nrounds; ++round) {
-        for (int64_t t = 0; t < ntiles; ++t, ++it) {
+        int64_t nt = ntiles, lo = 0;
+        if (LISTED) { const int64_t u = unit_of(round); lo = list_lo(u); nt = list_len(u); }
+        for (int64_t t = 0; t < nt; ++t, ++it) {
           const int s = (int)(it % NS);
           const uint32_t ph = (uint32_t)((it / NS) & 1);
           if (p.sync_ctr != nullptr && (it % TC_SYNC_EVERY) == 0) {
@@ -461,7 +479,8 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
           }
           mbar_wait(empty_b + 8 * s, ph ^ 1);      // every CTA of the cluster has consumed this stage
           mbar_arrive_expect_tx(full_b + 8 * s, NPART * sizeB);
-          const int row0 = (int)(btile(round, t) * TC_N) + (int)crank * ROWS;
+          const int64_t tile = LISTED ? (int64_t)p.unit_tiles[lo + t] : btile(round, t);
+          const int row0 = (int)(tile * TC_N) + (int)crank * ROWS;
           for (int part = 0; part < NPART; ++part) {
             const CUtensorMap* mm = part ? &mBl : &mBh;
             const CUtensorMap* mt = part ? &mBlt : &mBht;
@@ -498,7 +517,8 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
     for (int64_t round = 0; round < nrounds; ++round) {
     mbar_wait(bar_a, (uint32_t)(round & 1));   // this round's A rows stored to TMEM by the epilogue warps
     tc_fence_after();
-    for (int64_t tile = 0; tile < ntiles; ++tile, ++it) {
+    const int64_t nt = LISTED ? list_len(unit_of(round)) : ntiles;
+    for (int64_t tile = 0; tile < nt; ++tile, ++it) {
       const int s = (int)(it % NS);            // shared-memory stage
       const uint32_t ph = (uint32_t)((it / NS) & 1);
       mbar_wait(full_b + 8 * s, ph);
@@ -560,7 +580,10 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
     const int my_qt = (QT == 2) ? grp : 0;
     const int lgrp = (QT == 2) ? 0 : grp;            // list index inside a row's candidate storage
     const uint32_t a_col0 = (uint32_t)(my_qt * 64);
+    int64_t it_run = 0;                              // LISTED: tiles of the earlier rounds (lists differ in length)
     for (int64_t round = 0; round < nrounds; ++round) {
+    int64_t nt = ntiles, lo = 0;
+    if (LISTED) { const int64_t u = unit_of(round); lo = list_lo(u); nt = list_len(u); }
     const int64_t q0 = q0_of(round, my_qt);
     const int64_t gq = q0 + row;
     const bool valid = gq < p.nq;
@@ -620,10 +643,11 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
 
     // this group's tiles.  QT == 1: running iteration index it = round * ntiles + t with it % 2 == grp; QT == 2:
     // every tile, accumulator index 2 it + grp
-    const int64_t it0 = round * ntiles;
-    for (int64_t t = (QT == 2) ? 0 : ((grp + (it0 & 1)) & 1); t < ntiles; t += (QT == 2 ? 1 : TC_GROUPS)) {
+    const int64_t it0 = LISTED ? it_run : round * ntiles;
+    if (LISTED) it_run += nt;
+    for (int64_t t = (QT == 2) ? 0 : ((grp + (it0 & 1)) & 1); t < nt; t += (QT == 2 ? 1 : TC_GROUPS)) {
       const int64_t it = it0 + t;
-      const int64_t tile = btile(round, t);
+      const int64_t tile = LISTED ? (int64_t)p.unit_tiles[lo + t] : btile(round, t);
       const int64_t ait = (QT == 2) ? (it * 2 + grp) : it;
       const int s = (int)(ait % NA);                   // accumulator of this iteration
       const uint32_t ph = (uint32_t)((ait / NA) & 1);
@@ -1001,9 +1025,11 @@ int launch_tc_cl(const void* q_hi, const void* q_lo, const void* r_hi, const voi
   int64_t rem_units = 0, piece_k = 0, piece_tpp = 0;
   uint2* piece_space = p.piece_buf;
   p.q_unit0 = 0; p.split_k = 0;
+  const bool listed = p.unit_ptr != nullptr;
+  p.n_units = n_cluster_tiles;
   if constexpr (MODE == 0 && FMT == 3 && !WIDE) {
     const int64_t full = n_cluster_tiles / n_clusters, rem = n_cluster_tiles % n_clusters;
-    if (piece_space != nullptr && full >= 1 && rem > 0 && rem * 2 <= n_clusters && total_tiles >= 64) {
+    if (!listed && piece_space != nullptr && full >= 1 && rem > 0 && rem * 2 <= n_clusters && total_tiles >= 64) {
       int64_t k = n_clusters / rem;
       if (k > TC_SPLIT_MAX) k = TC_SPLIT_MAX;
       piece_tpp = gtb_cdiv(total_tiles, k);
@@ -1016,7 +1042,7 @@ int launch_tc_cl(const void* q_hi, const void* q_lo, const void* r_hi, const voi
   }
   const unsigned nblk = (unsigned)(n_clusters * CL);
   // pacing counter: one caller-owned device word, zeroed per launch (no state is kept in the library)
-  if (p.sync_ctr != nullptr && nblk > (unsigned)CL && splits == 1) {
+  if (p.sync_ctr != nullptr && nblk > (unsigned)CL && splits == 1 && !listed) {
     GTB_CUDA(cudaMemsetAsync(p.sync_ctr, 0, sizeof(unsigned int), st));
   } else {
     p.sync_ctr = nullptr;
@@ -1033,6 +1059,15 @@ int launch_tc_cl(const void* q_hi, const void* q_lo, const void* r_hi, const voi
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
+  if constexpr (MODE == 0 && FMT == 3 && !WIDE) {
+    if (listed) {
+      auto lkern = search_tc_kernel<MODE, CL, FMT, LS, QT, false, false, true>;
+      GTB_CUDA(cudaFuncSetAttribute(lkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      GTB_CUDA(cudaLaunchKernelEx(&cfg, lkern, mBh, mBht, mBl, mBlt, q_hi, q_lo, p));
+      GTB_CHECK_LAUNCH();
+      return GTB_OK;
+    }
+  }
   GTB_CUDA(cudaLaunchKernelEx(&cfg, kern, mBh, mBht, mBl, mBlt, q_hi, q_lo, p));
   GTB_CHECK_LAUNCH();
   if constexpr (MODE == 0 && FMT == 3 && !WIDE) {
@@ -1220,13 +1255,19 @@ static int tc_check(int64_t nq, int64_t nr, int64_t nq_pad, int64_t nr_pad, int 
 extern "C" int gtb_knn_topk_tc_seeded(const void* q_hi, const void* q_lo, const float* qn2, int64_t nq, int64_t nq_pad,
                                       const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp, int dtype,
                                       int list, int cluster, int qtiles, const float* seed_tau, int tile_stride,
-                                      int32_t* cand_idx, void* scratch, float* tau, unsigned int* pace, void* stream) {
+                                      int32_t* cand_idx, void* scratch, float* tau, unsigned int* pace,
+                                      const int64_t* unit_ptr, const int32_t* unit_tiles, const int32_t* unit_order,
+                                      void* stream) {
   int rc = tc_check(nq, nr, nq_pad, nr_pad, Kp, dtype);
   if (rc) return rc;
   GTB_CHECK_ARG(list == 16 || list == 32, "list size must be 16 or 32");
   GTB_CHECK_ARG(qtiles == 1 || qtiles == 2, "query tiles per CTA: 1 or 2");
   GTB_CHECK_ARG(tile_stride >= 1, "tile_stride must be >= 1");
+  const bool listed = unit_ptr != nullptr || unit_tiles != nullptr || unit_order != nullptr;
+  GTB_CHECK_ARG(!listed || (unit_ptr && unit_tiles && unit_order), "tile lists need unit_ptr, unit_tiles and unit_order");
+  GTB_CHECK_ARG(!listed || (dtype == 3 && tile_stride == 1), "tile lists: the one-product flavour (dtype 3), tile_stride 1");
   TcParams p{};
+  p.unit_ptr = unit_ptr; p.unit_tiles = unit_tiles; p.unit_order = unit_order;
   p.nq = nq; p.nq_pad = nq_pad; p.nr = nr; p.nr_pad = nr_pad; p.qn2 = qn2;
   p.cand_idx = cand_idx; p.cand_buf = reinterpret_cast<uint2*>(scratch); p.tau = tau; p.sync_ctr = pace;
   p.seed_tau = seed_tau; p.tile_stride = tile_stride;
@@ -1255,7 +1296,7 @@ extern "C" int gtb_knn_topk_tc(const void* q_hi, const void* q_lo, const float* 
                                int list, int cluster, int qtiles, int32_t* cand_idx, void* scratch, float* tau,
                                unsigned int* pace, void* stream) {
   return gtb_knn_topk_tc_seeded(q_hi, q_lo, qn2, nq, nq_pad, r_hi, r_lo, nr, nr_pad, Kp, dtype, list, cluster, qtiles,
-                                nullptr, 1, cand_idx, scratch, tau, pace, stream);
+                                nullptr, 1, cand_idx, scratch, tau, pace, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" int gtb_knn_radius_tc(const void* q_hi, const void* q_lo, const float* qn2, const float* lim2,

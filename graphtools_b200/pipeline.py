@@ -248,6 +248,7 @@ class SearchOperand:
         self._n2_tc = None
         self._maxnorm = None
         self._maxnorm_host = None
+        self._perm = None
 
     # -- CUDA-core operand: k-major [d_pad][n_pad] + norms
     def simt(self):
@@ -317,6 +318,27 @@ class SearchOperand:
             self._maxnorm = mx
             self._n2_tc = n2
         return self.maxnorm
+
+    def locality_order(self):
+        """perm (int32 [n]): the rows grouped by nearest of ORDER_PIVOTS pivot rows, stable (csrc/order.cu) -- consecutive
+        rows of the order lie close together, so a 128-row tile of them covers one region of the data."""
+        if self._perm is None:
+            P = min(ORDER_PIVOTS, self.n)
+            cell = _empty((self.n,), torch.int32)
+            E.call("gtb_order_assign", self.Xs, self.n, self.d, P, cell)
+            ws = _empty((E.lib().gtb_order_ws_elems(self.n, P),), torch.int32)
+            self._perm = _empty((self.n,), torch.int32)
+            E.call("gtb_order_sort", cell, self.n, P, ws, self._perm)
+        return self._perm
+
+    def geometry(self, rows):
+        """(centroids float64 [d][g], radii float64 [g]) of the groups of ``rows`` consecutive rows of the locality order,
+        over ``X`` (the rows the exact stage reads); g = n_pad / rows rounded up, radius -1 for a group without rows."""
+        g = -(-self.n_pad // rows)
+        cent = _empty((self.d, g), torch.float64)
+        rad = _empty((g,), torch.float64)
+        E.call("gtb_tile_geometry", self.X, self.n, self.d, int(self.is64), self.locality_order(), rows, g, cent, rad)
+        return cent, rad
 
     @property
     def maxnorm(self):
@@ -498,6 +520,8 @@ FALLBACK = {"auto": (AUTO_TC, "tch", "tc16", "tc", "simt"), "tc": ("tc", "tc16",
             "tch": ("tch", "tc16", "tc", "simt"), "tch1": ("tch1", "tch", "tc16", "tc", "simt"), "simt": ("simt",)}
 TC_CLUSTER = 2           # CTAs per cluster sharing each reference tile by TMA multicast
 SEED_STRIDE = 16         # the seed sweep of the one-product flavour visits every 16th reference tile
+ORDER_PIVOTS = 256       # cells of the locality order of the pruned sweep
+PRUNE_MAX_VISITED = 0.5  # the pruned sweep runs when its tile lists hold at most this share of all (unit, tile) pairs
 SearchPlan = namedtuple("SearchPlan", "impl ls qtiles S ntau seeded")
 
 
@@ -536,6 +560,62 @@ def plan_search(want, d, n_pad, metric, knn, kmax, binary):
     return SearchPlan(impl, ls, qtiles, 2 * ls, 2, f.dtype == 3 and seedable)
 
 
+def prunable(plan, metric):
+    """Whether a search tries the pruned sweep (tile lists over locality-ordered operands): the seeded one-product
+    flavour under a metric whose exact stage reads the rows the tile geometry is computed from.  (Cosine and correlation
+    search a normalised copy whose rounding the bound does not cover.)"""
+    return plan.impl == "tch1" and plan.seeded and metric in ("euclidean", "sqeuclidean")
+
+
+def use_tile_lists(visited, total):
+    """The pruned sweep, or the plain seeded sweep when the lists visit more than PRUNE_MAX_VISITED of all (unit, tile)
+    pairs (isotropic data, no region holds a unit's neighbourhood): the listed sweep gives up the grid-wide pacing that
+    lets every reference tile be read from DRAM once."""
+    return 0 < total and visited <= PRUNE_MAX_VISITED * total
+
+
+def unit_bounds(seed, qn2, eps_rel, maxnorm, s2, unit_rows, n_units):
+    """T_U (float64 [n_units]): per unit of ``unit_rows`` consecutive query rows, the largest seed + E of its rows in data
+    units -- ``seed`` [nq, >= 1] the sweep's starting thresholds (scaled squared distances, slot 0), ``qn2`` [nq] the
+    rows' squared norms, E = eps_rel (qn2 + maxnorm) the certified rounding bound of the sweep, widened by 2^-20
+    (qn2 + maxnorm) for the float32 rounding of threshold - |x|^2 in the sweep.  A reference point at exact squared
+    distance >= T_U from a row of the unit has approximate distance >= the row's seed, so the sweep would never admit
+    it: skipping it leaves the candidate lists as they were.  Units without rows: -inf."""
+    t = seed[:, 0].to(torch.float64) / s2 + (eps_rel + 2.0 ** -20) * (qn2.to(torch.float64) + maxnorm)
+    out = torch.full((n_units * unit_rows,), -math.inf, dtype=torch.float64, device=seed.device)
+    out[:t.shape[0]] = t
+    return out.view(n_units, unit_rows).amax(dim=1)
+
+
+def _tile_lists(qry, ref, seed, q_n2, eps_rel, s2, unit_rows):
+    """Reference tile lists of the query units (csrc/order.cu) over the locality orders of both operands.  Returns
+    (visited, total, lists) with lists = (unit_ptr, unit_tiles, unit_order) or None when use_tile_lists declines."""
+    nt = ref.n_pad // 128
+    n_units = -(-qry.n_pad // unit_rows)
+    rc, rr = ref.geometry(128)
+    uc, ur = qry.geometry(unit_rows)
+    pq = qry.locality_order().long()
+    ub = unit_bounds(seed.index_select(0, pq), q_n2[:qry.n].index_select(0, pq), eps_rel, ref.maxnorm, s2, unit_rows,
+                     n_units)
+    keep = _empty((n_units, nt), torch.uint8)
+    count = _empty((n_units,), torch.int32)
+    E.call("gtb_tile_lists_count", uc, ur, ub, n_units, rc, rr, nt, ref.d, keep, count)
+    ptr = exclusive_scan(count)
+    visited, total = int(ptr[-1].item()), n_units * nt
+    if not use_tile_lists(visited, total):
+        return visited, total, None
+    tiles = _empty((max(visited, 1),), torch.int32)
+    E.call("gtb_tile_lists_fill", keep, n_units, nt, ptr, tiles)
+    order = torch.argsort(count, descending=True, stable=True).to(torch.int32)   # longest lists first
+    return visited, total, (ptr, tiles, order)
+
+
+def _permuted_rows(t, perm, n):
+    """Rows of ``t`` [n_pad, ...] in the locality order; padding rows stay in place."""
+    idx = torch.cat([perm.long(), torch.arange(n, t.shape[0], device=t.device)])
+    return t.index_select(0, idx)
+
+
 def _sweep_tc(plan, qry, ref):
     """Tensor-core sweep: (candidates, tau, query norms, eps_rel, fp16 scale)."""
     f = FLAVOURS[plan.impl]
@@ -561,8 +641,28 @@ def _sweep_tc(plan, qry, ref):
             seed = _empty((nq, plan.ntau), torch.float32)
             E.call("gtb_knn_seed_tc", q_hi, qn2_s, nq, qry.n_pad, r_hi, ref.n, ref.n_pad, Kp, TC_CLUSTER, SEED_STRIDE,
                    seed, pace)
-        E.call("gtb_knn_topk_tc_seeded", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, ref.n, ref.n_pad, Kp, f.dtype,
-               plan.ls, TC_CLUSTER, plan.qtiles, seed, 1, cand, scratch, tau, pace)
+        lists = None
+        _STATS.update(tile_pairs_visited=None)
+        if prunable(plan, ref.metric):
+            # pruned sweep: both operands in locality order, every unit (the TC_CLUSTER x 2 query tiles of one cluster
+            # round) sweeps only the reference tiles its seeds can reach; the lists come back in original row ids
+            visited, total, lists = _tile_lists(qry, ref, seed, q_n2, f.eps_rel(ref.d), s2, TC_CLUSTER * plan.qtiles * 128)
+            _STATS.update(tile_pairs_visited=visited / total)
+        _STATS.update(tile_lists=lists is not None)
+        if lists is None:
+            E.call("gtb_knn_topk_tc_seeded", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, ref.n, ref.n_pad, Kp,
+                   f.dtype, plan.ls, TC_CLUSTER, plan.qtiles, seed, 1, cand, scratch, tau, pace)
+        else:
+            perm_q, perm_r = qry.locality_order(), ref.locality_order()
+            pq_hi = _permuted_rows(q_hi, perm_q, nq)
+            pr_hi = _permuted_rows(r_hi, perm_r, ref.n)
+            cand_p = _empty((nq, plan.S), torch.int32)
+            tau_p = _empty((nq, plan.ntau), torch.float32)
+            # (the one-product flavour reads the hi arrays only)
+            E.call("gtb_knn_topk_tc_seeded", pq_hi, pq_hi, _permuted_rows(qn2_s, perm_q, nq), nq, qry.n_pad, pr_hi,
+                   pr_hi, ref.n, ref.n_pad, Kp, f.dtype, plan.ls, TC_CLUSTER, plan.qtiles,
+                   seed.index_select(0, perm_q.long()), 1, cand_p, scratch, tau_p, None, *lists)
+            E.call("gtb_unpermute_candidates", cand_p, tau_p, nq, plan.S, plan.ntau, perm_q, perm_r, cand, tau)
     else:
         E.call("gtb_knn_topk_tc", q_hi, q_lo, qn2_s, nq, qry.n_pad, r_hi, r_lo, ref.n, ref.n_pad, Kp, f.dtype, plan.ls,
                TC_CLUSTER, plan.qtiles, cand, scratch, tau, pace)

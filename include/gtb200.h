@@ -104,11 +104,16 @@ int gtb_knn_topk_tc(const void* q_hi, const void* q_lo, const float* qn2, int64_
  * slot 0 read): the row's threshold starts at the seed instead of +inf, every reference point under it is kept
  * (compacting to the list length when the buffer fills) and a list that never filled reports the seed as its tau -- a
  * seed from gtb_knn_seed_tc removes most of the list * ln(N / list) threshold updates of a cold start.
- * seed_tau = NULL, tile_stride = 1 is gtb_knn_topk_tc. */
+ * seed_tau = NULL, tile_stride = 1 is gtb_knn_topk_tc.  (d) tile lists (dtype 3, tile_stride 1; all three or none):
+ * unit u = the cluster * qtiles query tiles of rows [u * cluster * qtiles * 128, ...), u < cdiv(nq_pad / 128,
+ * cluster * qtiles), sweeps only the reference tiles unit_tiles[unit_ptr[u] .. unit_ptr[u + 1]); unit_order lists every
+ * unit once, in the order the clusters take them (longest list first balances the rounds); pace is not used.  A row's
+ * list and tau then cover the listed tiles only. */
 int gtb_knn_topk_tc_seeded(const void* q_hi, const void* q_lo, const float* qn2, int64_t nq, int64_t nq_pad,
                            const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp, int dtype,
                            int list, int cluster, int qtiles, const float* seed_tau, int tile_stride,
-                           int32_t* cand_idx, void* scratch, float* tau, unsigned int* pace, void* stream);
+                           int32_t* cand_idx, void* scratch, float* tau, unsigned int* pace,
+                           const int64_t* unit_ptr, const int32_t* unit_tiles, const int32_t* unit_order, void* stream);
 /* Threshold seeds (one-product float16 sweep over every tile_stride-th reference tile, no candidate lists): tau[nq][2]
  * (both slots) = the gtb_knn_seed_k()-th smallest TILE MINIMUM of the approximate squared distances, an upper bound of
  * the k-th smallest sampled value kept in registers by a branch-free insertion network -- no hit servicing at all */
@@ -116,6 +121,25 @@ int gtb_knn_seed_k(void);
 int gtb_knn_seed_tc(const void* q_hi, const float* qn2, int64_t nq, int64_t nq_pad, const void* r_hi, int64_t nr,
                     int64_t nr_pad, int Kp, int cluster, int tile_stride, float* tau, unsigned int* pace, void* stream);
 int64_t gtb_tc_scratch_bytes(int64_t nq_pad);
+/* Locality order and tile lists for the listed sweep (csrc/order.cu).  d <= 128 throughout.
+ * gtb_order_assign: cell[r] = nearest of the P (<= 512, <= n) pivot rows p * floor(n / P) of X (float32).
+ * gtb_order_sort: perm[i] = row at position i of the stable sort of the rows by cell; ws: gtb_order_ws_elems int32.
+ * gtb_tile_geometry: per group g of the rows perm[g * rows .. min(n, (g + 1) * rows)) of X (float64 if x64, else
+ * float32): centroid cent[k * ngroups + g] (float64) and radius rad[g] = max |x - c| rounded up (-1: no rows).
+ * gtb_tile_lists_count: keep[u * nt + t] = 0 iff (|c_u - c_t| - r_u - r_t)^2 >= ub[u] (rounded against skipping), every
+ * distance between the rows of unit u and tile t then reaching ub[u]; count[u] = kept tiles.
+ * gtb_tile_lists_fill: tiles[ptr[u] ..] = the kept tiles of unit u, ascending (ptr = exclusive scan of count).
+ * gtb_unpermute_candidates: cand[perm_q[i]][s] = perm_r[cand_p[i][s]] (-1 stays), tau[perm_q[i]] = tau_p[i]. */
+int gtb_order_assign(const float* X, int64_t n, int d, int P, int32_t* cell, void* stream);
+int64_t gtb_order_ws_elems(int64_t n, int P);
+int gtb_order_sort(const int32_t* cell, int64_t n, int P, int32_t* ws, int32_t* perm, void* stream);
+int gtb_tile_geometry(const void* X, int64_t n, int d, int x64, const int32_t* perm, int64_t rows, int64_t ngroups,
+                      double* cent, double* rad, void* stream);
+int gtb_tile_lists_count(const double* uc, const double* ur, const double* ub, int64_t nu, const double* rc,
+                         const double* rr, int64_t nt, int d, uint8_t* keep, int32_t* count, void* stream);
+int gtb_tile_lists_fill(const uint8_t* keep, int64_t nu, int64_t nt, const int64_t* ptr, int32_t* tiles, void* stream);
+int gtb_unpermute_candidates(const int32_t* cand_p, const float* tau_p, int64_t nq, int S, int ntau,
+                             const int32_t* perm_q, const int32_t* perm_r, int32_t* cand, float* tau, void* stream);
 int gtb_knn_radius_tc(const void* q_hi, const void* q_lo, const float* qn2, const float* lim2, int64_t nq,
                       int64_t nq_pad, const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp,
                       int dtype, int cluster, int32_t* pairs, int64_t capacity, unsigned long long* counter,
