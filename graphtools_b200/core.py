@@ -595,6 +595,25 @@ class BaseGraph(Base, metaclass=abc.ABCMeta):
         from . import paths
         return paths.shortest_path(self, method=method, distance=distance)
 
+    def diffusion_eigs(self, k=10, tol=1e-8, maxiter=None, random_state=None):
+        """The k largest eigenvalues ``w`` (float64 [k], descending) of the diffusion operator P = D^-1 K and its
+        right eigenvectors ``psi`` (float64 [N, k]): ``psi = D^-1/2 phi`` with ``phi`` orthonormal eigenvectors of
+        ``diff_aff``, so ``psi.T @ (D psi) = I`` for D = ``kernel_degree``; the entry of largest magnitude in every
+        column of ``psi`` is positive.  Every pair satisfies ``||diff_aff phi_i - w_i phi_i||_2 <= tol`` (relative:
+        ||diff_aff||_2 = 1).  Dense kernels and landmark graphs use their full kernel K.  The same ``random_state``
+        gives bit-identical results.  Raises ValueError for kernel_symm=None, k outside [1, N) or a row of zero
+        degree, and ``eigen.NoConvergence`` after ``maxiter`` outer iterations.  Runs on the device (eigen.py,
+        Chebyshev-filtered subspace iteration through csrc/spmm.cu)."""
+        from . import eigen
+        return eigen.diffusion_eigs(self, k=k, tol=tol, maxiter=maxiter, random_state=random_state)
+
+    def diffusion_map(self, n_components=2, t=1, tol=1e-8, maxiter=None, random_state=None):
+        """Diffusion-map embedding [N, n_components]: ``psi[:, 1:n+1] * w[1:n+1] ** t`` from
+        ``diffusion_eigs(n_components + 1)``, the stationary first pair dropped (Coifman & Lafon); t >= 0."""
+        from . import eigen
+        return eigen.diffusion_map(self, n_components=n_components, t=t, tol=tol, maxiter=maxiter,
+                                   random_state=random_state)
+
     @staticmethod
     def _materialize(dev):
         if isinstance(dev, pipeline.DeviceCSR):

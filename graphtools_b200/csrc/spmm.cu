@@ -12,6 +12,13 @@
 // Layout: one warp per output row; lane l owns columns {2l, 2l+1} of every 64-column chunk (double2 loads:
 // 512 contiguous bytes per warp and chunk).  Entries are consumed four at a time so that four independent row
 // gathers are in flight per warp.
+//
+// The same body, instantiated with the Chebyshev epilogue, is the filter step of the diffusion-map eigensolver
+// (eigen.py): out = (alpha (A . Y) + beta Y) + gamma Z, each product and sum rounded separately, i.e. numpy's
+// `alpha*S + beta*Y + gamma*Z` after scipy's S = A.dot(Y).  At the solver's block widths (16-32 columns) a whole
+// warp per row would leave most lanes idle, so that entry point gives each row the smallest power-of-two group of
+// LPR lanes that covers its columns two per lane, and packs 32 / LPR rows into a warp.  Algorithmic bytes per call:
+// nnz (12 + 8b) + 8 N (3b + 1) -- CSR, row gathers, the own rows of Y and Z, the write, indptr.
 #include "common.cuh"
 #include "gtb200.h"
 
@@ -20,14 +27,17 @@ namespace {
 constexpr int SPMM_WARPS = 8;
 constexpr int SPMM_UNROLL = 4;
 
-// NCH = 64-column chunks held in registers by one warp pass (f <= 64 * NCH handled in one sweep over the row)
-template <int NCH>
+// NCH = chunks of 2 LPR columns held in registers by one pass of a row's LPR-lane group (f <= 2 LPR NCH handled in
+// one sweep over the row).  CHEB adds the epilogue (alpha s + beta B[row]) + gamma Z[row]; B is then square-indexed
+// (Y) and Z may alias out: every element of Z is read only by the thread that writes that element of out.
+template <int NCH, int LPR, bool CHEB>
 __global__ void __launch_bounds__(SPMM_WARPS * 32)
 spmm_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ idx, const double* __restrict__ val,
-                int64_t n_rows, const double* __restrict__ B, int64_t ldb, int f, int col0, double* __restrict__ out,
-                int64_t ldo) {
-  const int lane = threadIdx.x & 31;
-  const int64_t row = (int64_t)blockIdx.x * SPMM_WARPS + (threadIdx.x >> 5);
+                int64_t n_rows, const double* __restrict__ B, int64_t ldb, int f, int col0, double* out,
+                int64_t ldo, double alpha, double beta, double gamma, const double* Z, int64_t ldz) {
+  constexpr int CW = 2 * LPR;                      // columns per chunk
+  const int lane = threadIdx.x & (LPR - 1);
+  const int64_t row = (int64_t)blockIdx.x * (SPMM_WARPS * 32 / LPR) + (threadIdx.x / LPR);
   if (row >= n_rows) return;
   const int64_t p0 = indptr[row], p1 = indptr[row + 1];
   double ax[NCH], ay[NCH];
@@ -35,7 +45,7 @@ spmm_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ 
 #pragma unroll
   for (int c = 0; c < NCH; ++c) {
     ax[c] = 0.0; ay[c] = 0.0;
-    const int k = col0 + c * 64 + 2 * lane;
+    const int k = col0 + c * CW + 2 * lane;
     okx[c] = k < f; oky[c] = k + 1 < f;
   }
   const bool vec = ((ldb & 1) == 0) && ((reinterpret_cast<uintptr_t>(B) & 15) == 0);
@@ -56,11 +66,11 @@ spmm_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ 
         bx[u][c] = 0.0; by[u][c] = 0.0;
         if (p + u < p1) {
           if (vec && oky[c]) {
-            const double2 t = *reinterpret_cast<const double2*>(src[u] + c * 64);
+            const double2 t = *reinterpret_cast<const double2*>(src[u] + c * CW);
             bx[u][c] = t.x; by[u][c] = t.y;
           } else {
-            if (okx[c]) bx[u][c] = src[u][c * 64];
-            if (oky[c]) by[u][c] = src[u][c * 64 + 1];
+            if (okx[c]) bx[u][c] = src[u][c * CW];
+            if (oky[c]) by[u][c] = src[u][c * CW + 1];
           }
         }
       }
@@ -77,11 +87,32 @@ spmm_csr_kernel(const int64_t* __restrict__ indptr, const int32_t* __restrict__ 
     }
   }
   double* o = out + row * ldo + col0 + 2 * lane;
+  if constexpr (CHEB) {
+    const double* y = B + row * ldb + col0 + 2 * lane;
+    const double* z = Z + row * ldz + col0 + 2 * lane;
+#pragma unroll
+    for (int c = 0; c < NCH; ++c) {
+      if (okx[c])
+        ax[c] = __dadd_rn(__dadd_rn(__dmul_rn(alpha, ax[c]), __dmul_rn(beta, y[c * CW])), __dmul_rn(gamma, z[c * CW]));
+      if (oky[c])
+        ay[c] = __dadd_rn(__dadd_rn(__dmul_rn(alpha, ay[c]), __dmul_rn(beta, y[c * CW + 1])),
+                          __dmul_rn(gamma, z[c * CW + 1]));
+    }
+  }
 #pragma unroll
   for (int c = 0; c < NCH; ++c) {
-    if (okx[c]) o[c * 64] = ax[c];
-    if (oky[c]) o[c * 64 + 1] = ay[c];
+    if (okx[c]) o[c * CW] = ax[c];
+    if (oky[c]) o[c * CW + 1] = ay[c];
   }
+}
+
+template <int LPR>
+void launch_cheb(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const double* Y, int64_t ldy,
+                 int f, double alpha, double beta, double gamma, const double* Z, int64_t ldz, double* out,
+                 int64_t ldo, cudaStream_t st) {
+  const unsigned grid = (unsigned)gtb_cdiv(n, SPMM_WARPS * 32 / LPR);
+  spmm_csr_kernel<1, LPR, true><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n, Y, ldy, f, 0, out, ldo, alpha,
+                                                                 beta, gamma, Z, ldz);
 }
 
 // out[i][k] *= s[i]  /  out[i][k] = in[i][k] * s[i]   (row scaling used around the SpMM for D^-1/2 K D^-1/2 products)
@@ -104,11 +135,51 @@ extern "C" int gtb_spmm_csr(const int64_t* indptr, const int32_t* idx, const dou
   const unsigned grid = (unsigned)gtb_cdiv(n_rows, SPMM_WARPS);
   for (int col0 = 0; col0 < f; col0 += 128) {
     if (f - col0 > 64)
-      spmm_csr_kernel<2><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n_rows, B, ldb, f, col0, out, ldo);
+      spmm_csr_kernel<2, 32, false><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n_rows, B, ldb, f, col0, out,
+                                                                     ldo, 0.0, 0.0, 0.0, nullptr, 0);
     else
-      spmm_csr_kernel<1><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n_rows, B, ldb, f, col0, out, ldo);
+      spmm_csr_kernel<1, 32, false><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n_rows, B, ldb, f, col0, out,
+                                                                     ldo, 0.0, 0.0, 0.0, nullptr, 0);
     GTB_CHECK_LAUNCH();
   }
+  return GTB_OK;
+}
+
+extern "C" int gtb_spmm_cheb(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n,
+                             const double* Y, int64_t ldy, int f, double alpha, double beta, double gamma,
+                             const double* Z, int64_t ldz, double* out, int64_t ldo, void* stream) {
+  GTB_CHECK_ARG(n > 0 && f > 0 && ldy >= f && ldz >= f && ldo >= f, "bad shape");
+  GTB_CHECK_ARG(Y != nullptr && Z != nullptr && out != nullptr, "null operand");
+  // out overlapping Y would overwrite rows other threads still gather.  out may be Z itself (same pointer, same
+  // leading dimension: every element of Z is then read only by the thread that writes it); any other overlap with
+  // Z would let one thread's write land on an element another thread still reads.
+  const uintptr_t o0 = reinterpret_cast<uintptr_t>(out), o1 = o0 + (uintptr_t)(((n - 1) * ldo + f) * sizeof(double));
+  const uintptr_t y0 = reinterpret_cast<uintptr_t>(Y), y1 = y0 + (uintptr_t)(((n - 1) * ldy + f) * sizeof(double));
+  const uintptr_t z0 = reinterpret_cast<uintptr_t>(Z), z1 = z0 + (uintptr_t)(((n - 1) * ldz + f) * sizeof(double));
+  GTB_CHECK_ARG(o1 <= y0 || y1 <= o0, "out must not overlap Y");
+  GTB_CHECK_ARG((o0 == z0 && ldo == ldz) || o1 <= z0 || z1 <= o0, "out must be Z itself or not overlap it");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (f > 64) {
+    const unsigned grid = (unsigned)gtb_cdiv(n, SPMM_WARPS);
+    for (int col0 = 0; col0 < f; col0 += 128) {
+      if (f - col0 > 64)
+        spmm_csr_kernel<2, 32, true><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n, Y, ldy, f, col0, out, ldo,
+                                                                      alpha, beta, gamma, Z, ldz);
+      else
+        spmm_csr_kernel<1, 32, true><<<grid, SPMM_WARPS * 32, 0, st>>>(indptr, idx, val, n, Y, ldy, f, col0, out, ldo,
+                                                                      alpha, beta, gamma, Z, ldz);
+      GTB_CHECK_LAUNCH();
+    }
+    return GTB_OK;
+  }
+  const int lanes = (f + 1) / 2;                 // smallest power-of-two group with at least ceil(f / 2) lanes
+  if (lanes <= 1)       launch_cheb<1>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  else if (lanes <= 2)  launch_cheb<2>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  else if (lanes <= 4)  launch_cheb<4>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  else if (lanes <= 8)  launch_cheb<8>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  else if (lanes <= 16) launch_cheb<16>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  else                  launch_cheb<32>(indptr, idx, val, n, Y, ldy, f, alpha, beta, gamma, Z, ldz, out, ldo, st);
+  GTB_CHECK_LAUNCH();
   return GTB_OK;
 }
 

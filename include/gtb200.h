@@ -292,6 +292,15 @@ int gtb_dense_rowsum(const double* K, int64_t nq, int64_t nr, double* sum, void*
  * accumulated in stored order with separate multiply and add (bit-identical to scipy's A.dot(B)) */
 int gtb_spmm_csr(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n_rows, const double* B,
                  int64_t ldb, int f, double* out, int64_t ldo, void* stream);
+/* Chebyshev filter step of the diffusion-map eigensolver (graphtools_b200/eigen.py): out[n][ldo] (first f columns)
+ * = (alpha (A . Y) + beta Y) + gamma Z for a square CSR float64 A [n x n] and row-major float64 Y, Z.  A . Y is
+ * accumulated as gtb_spmm_csr does and every product and sum of the epilogue is rounded separately, so the result
+ * is bit-identical to scipy's S = A.dot(Y) followed by numpy's alpha*S + beta*Y + gamma*Z.  out may be Z itself
+ * (same pointer, ldo == ldz: the three-term recurrence rotates two buffers); out overlapping Y, or overlapping Z
+ * in any other way, is rejected (GTB_ERR_ARG). */
+int gtb_spmm_cheb(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const double* Y,
+                  int64_t ldy, int f, double alpha, double beta, double gamma, const double* Z, int64_t ldz,
+                  double* out, int64_t ldo, void* stream);
 /* out[i][:] = in[i][:] * s[i]   (power_neg_half = 0)   or   in[i][:] / sqrt(s[i])   (power_neg_half = 1) */
 int gtb_row_scale(const double* in, const double* s, int64_t n, int f, int power_neg_half, double* out,
                   void* stream);
