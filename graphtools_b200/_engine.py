@@ -45,6 +45,12 @@ _SIGS = {
     "gtb_unpermute_candidates": ([_P, _P, c_int64, c_int, c_int, _P, _P, _P, _P, _P], 1),
     "gtb_knn_radius_tc": ([_P, _P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, _P, c_int64,
                            _P, _P, _P, _P], 1),
+    "gtb_knn_count_tc": ([_P, _P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, c_int, c_int,
+                          c_int, _P, _P, _P], 1),
+    "gtb_knn_count_simt": ([_P, _P, _P, c_int64, c_int64, _P, _P, c_int64, c_int64, c_int, c_int, c_int, c_int, _P, _P],
+                           1),
+    "gtb_knn_count_bound": ([_P, _P, c_int64, c_int64, c_int, c_int, c_float, _P, c_float, c_double, c_int, c_int,
+                             c_int64, c_double, c_double, _P, c_int, c_double, _P, _P, _P, _P, _P], 1),
     "gtb_refine_topk": ([_P, c_int64, _P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_float, c_double, c_int, c_int64, c_double,
                          c_double, _P, c_int, c_double, _P, _P, _P, _P, _P, _P, _P, _P], 1),
     "gtb_compact_todo": ([_P, c_int64, _P, _P, _P], 1),

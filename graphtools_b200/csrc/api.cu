@@ -13,4 +13,4 @@ void gtb_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* gtb_last_error(void) { return g_err; }
-extern "C" int gtb_version(void) { return 204; }   // + gtb_spmm_cheb (Chebyshev filter step, csrc/spmm.cu)
+extern "C" int gtb_version(void) { return 205; }   // + gtb_knn_count_tc / _simt / _bound (knn beyond the lists)

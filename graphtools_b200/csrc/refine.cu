@@ -79,6 +79,10 @@ __device__ __forceinline__ double search2_of_key(double key, int metric) {
 __device__ __forceinline__ double search2_of_radius(double r, int metric) {
   return metric == 0 ? r * r : ((metric == 1 || metric == 4) ? 2.0 * r : r);
 }
+// inverse of search2_of_radius (rounded: callers widen the result)
+__device__ __forceinline__ double radius_of_search2(double s2, int metric) {
+  return metric == 0 ? sqrt(s2) : ((metric == 1 || metric == 4) ? 0.5 * s2 : s2);
+}
 
 // squared cosine distance between two rows of the ORIGINAL data, float64, one warp.  An all-zero row is at
 // distance 1 from every row, itself included: sklearn's normalize leaves it at zero, so its dot products are 0.
@@ -152,6 +156,24 @@ template <typename T>
 __device__ __forceinline__ double warp_metric2(const T* xq, double mq, const T* xr, int d, int lane, int metric) {
   if (metric == 4) return warp_corr2<T>(xq, mq, xr, d, lane);
   return metric == 1 ? warp_cos2<T>(xq, xr, d, lane) : warp_l1sq<T>(xq, xr, d, lane);
+}
+
+// The radius pass of a row the candidate list cannot finish.  Every reference point whose exact distance is <= the
+// returned radius must reach the row's ball.  dk: the knn-th distance, or an upper bound on it; bw: the row's bandwidth
+// (from dk when bw_mode == 0); bw_cert: bw is the row's true bandwidth -- otherwise bw is only an upper bound and the
+// ball must also hold the true knn nearest (radius >= dk), from which refine_ball_kernel recomputes it; dkmax: an upper
+// bound on the kmax-th distance (+inf: none), beyond which no neighbour is kept.
+__device__ __forceinline__ double collect_radius(const RowParams& rp, double dk, double bw, bool bw_cert, double dkmax) {
+  if (rp.decay < 0) return dk;
+  const double r = bw * rp.rfac;
+  return fmin(bw_cert ? r : fmax(r, dk), dkmax);
+}
+// Collect limit in search units, rounded up: search2 of the radius widened by 1e-6 (rounding of the radius itself), plus
+// the sweep's rounding bound E at the row (cityblock: plus its relative error at the radius).
+__device__ __forceinline__ float collect_limit(double r_search, int metric, double E, double eps_rel) {
+  double l2 = search2_of_radius(r_search, metric) * (1.0 + 1e-6) + E;
+  if (metric == 2) l2 += 2.0 * eps_rel * r_search;     // relative error at the radius, not at tau
+  return __double2float_ru(l2);
 }
 
 __device__ __forceinline__ int next_pow2(int x) {
@@ -448,12 +470,12 @@ __global__ void __launch_bounds__(R1_WARPS * 32, 6) refine_topk_kernel(Refine1Pa
                        ? p.eps_rel * fabs((double)tau) + (p.qn2 ? ((double)p.qn2[row] + (double)p.maxrn2) * 0x1p-23 : 0.0)
                        : p.eps_rel * ((double)p.qn2[row] + (double)p.maxrn2);
   const double rho2 = (double)tau - E;  // exact d2 of every non-candidate is >= rho2
-  double bw = 0.0, r_search = 0.0, dk = 0.0;
+  double bw = 0.0, dk = 0.0;
   bool done, bw_cert = true;
   if (rp.decay < 0) {
     double dk2 = key[rp.knn - 1];
     done = all_found || search2_of_key(dk2, rp.metric) < rho2;
-    r_search = sqrt(dk2);
+    dk = sqrt(dk2);
   } else {
     if (rp.bw_mode == 0) {
       double dk2 = key[rp.knn - 1];
@@ -467,19 +489,15 @@ __global__ void __launch_bounds__(R1_WARPS * 32, 6) refine_topk_kernel(Refine1Pa
     bool ball_cert = all_found || search2_of_radius(r, rp.metric) < rho2;
     bool kmax_cert = (rp.kmax <= (int64_t)n_cand) && search2_of_key(key[rp.kmax - 1], rp.metric) < rho2;
     done = bw_cert && (ball_cert || kmax_cert);
-    // an uncertified bandwidth is only an upper bound: the search ball must then also hold the
-    // true knn nearest (radius >= bw) so stage 2 can recompute it
-    r_search = bw_cert ? r : fmax(r, dk);
-    if (rp.kmax <= (int64_t)n_cand) r_search = fmin(r_search, sqrt(key[rp.kmax - 1]));
   }
+  const double dkmax = (rp.decay >= 0 && rp.kmax <= (int64_t)n_cand) ? sqrt(key[rp.kmax - 1]) : DBL_MAX * 2.0;
+  const double r_search = collect_radius(rp, dk, bw, bw_cert, dkmax);
   if (lane == 0) {
     p.bw_out[row] = bw;
     p.status[row] = done ? 1 : (bw_cert ? 0 : 2);
     p.nzero[row] = nz;
     if (!done) {
-      double l2 = search2_of_radius(r_search, rp.metric) * (1.0 + 1e-6) + E;
-      if (rp.metric == 2) l2 += 2.0 * p.eps_rel * r_search;     // relative error at the radius, not at tau
-      p.lim2_out[row] = __double2float_ru(l2);
+      p.lim2_out[row] = collect_limit(r_search, rp.metric, E, p.eps_rel);
       p.n_keep[row] = 0;
     } else {
       p.lim2_out[row] = 0.f;
@@ -655,6 +673,116 @@ __global__ void compact_todo_kernel(const int32_t* __restrict__ status, int64_t 
   if (todo) todo_rows[base + __popc(m & ((1u << lane) - 1))] = (int32_t)i;
 }
 
+// ------------------------------------------------------------------ bound selection from the count sweeps
+// Histograms of the approximate squared distances w (search units, the float32 values the sweep computes) from
+// gtb_knn_count_tc / gtb_knn_count_simt.  Coarse bin b < 63 holds w < 2^(elo + b - 126) (bin b > 0: w >= 2^(elo + b -
+// 127)), bin 63 everything above; the fine histogram splits the octave [t/2, t) below the coarse crossing edge t into
+// 16 sub-bins, bin 0 = everything under t/2.  Every edge is a power of two or a power of two times (1 + j/16): exact in
+// float32 and float64, so "count at edge" means exactly c(e) = #{w < e}.
+//
+// Why the bound holds: if c(e) >= k, then k reference points have w < e, hence exact squared distance < e + E (E the
+// sweep's rounding bound at the row, plus the float32 rounding of w = (|y|^2 - 2 x.y) + |x|^2), so the exact k-th
+// smallest squared distance is <= U = e + E.  A count that misses a point only moves the crossing up and U with it.
+// U bounds the knn-th distance from above exactly as the k-th candidate of an uncertified list does (status 2), so
+// collect_radius / collect_limit give the row's collect limit by the refine's own rule.
+struct BoundParams {
+  RowParams rp;
+  const uint32_t* coarse; const uint32_t* fine; int64_t nq; int elo, margin; float s2;
+  const float* qn2; float maxrn2; double eps_rel; int64_t nr;
+  float* top; float* lim2; int32_t* ball_lo; int32_t* ball_hi;
+};
+
+__device__ __forceinline__ float coarse_edge(int elo, int b) {     // upper edge of coarse bin b (+inf for bin 63)
+  return b >= 63 ? gtb_inf_f() : __uint_as_float((uint32_t)(elo + b + 1) << 23);
+}
+
+// first bin whose cumulative count reaches k (nb when none), cumulative counts before it and at it
+__device__ __forceinline__ int crossing(const uint32_t* h, int nb, int64_t k, int64_t* before) {
+  int64_t c = 0;
+  for (int b = 0; b < nb; ++b) {
+    if (c + h[b] >= k) { *before = c; return b; }
+    c += h[b];
+  }
+  *before = c;
+  return nb;
+}
+
+__global__ void count_bound_kernel(BoundParams p) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.nq) return;
+  const RowParams& rp = p.rp;
+  const int metric = rp.metric;
+  const double nrm = p.qn2 ? (double)p.qn2[i] + (double)p.maxrn2 : 0.0;
+  if (p.coarse == nullptr) {
+    // fixed bandwidth: the kernel support alone (status 0 of the refine), no count needed
+    const double bw = fmax((rp.bw_mode == 1 ? rp.bw_fixed[0] : rp.bw_fixed[i]) * rp.bw_scale, rp.bw_floor);
+    const double r = collect_radius(rp, 0.0, bw, true, DBL_MAX * 2.0);
+    const double E = metric == 2 ? nrm * 0x1p-23 : p.eps_rel * nrm;
+    p.lim2[i] = collect_limit(r, metric, E, p.eps_rel);
+    return;
+  }
+  const uint32_t* hc = p.coarse + i * 64;
+  int64_t before = 0;
+  const int bc = crossing(hc, 64, rp.knn, &before);
+  const float t = bc < 64 ? coarse_edge(p.elo, bc) : gtb_inf_f();
+  if (p.fine == nullptr) { p.top[i] = t; return; }
+  if (!(t < gtb_inf_f())) {
+    // fewer than k points under the window's top (fewer than k reference rows): every point is in the ball
+    p.lim2[i] = gtb_inf_f();
+    p.ball_lo[i] = (int32_t)p.nr; p.ball_hi[i] = (int32_t)p.nr;
+    return;
+  }
+  // fine crossing of k (and of kmax <= k): upper edge of the first sub-bin reaching it; t itself when the fine counts
+  // fall short (the coarse count at t already reaches k)
+  const uint32_t* hf = p.fine + i * 17;
+  auto fine_edge = [&](int64_t k) -> double {
+    int64_t c0 = 0;
+    const int b = crossing(hf, 17, k, &c0);
+    return b == 0 ? 0.5 * (double)t : (b < 17 ? 0.5 * (double)t * (1.0 + b / 16.0) : (double)t);
+  };
+  // search units -> data units (s2 is a power of two), plus the rounding bound
+  auto upper = [&](double e) {
+    e /= p.s2;
+    return metric == 2 ? e * (1.0 + p.eps_rel) + nrm * 0x1p-23 : e + (p.eps_rel + 0x1p-20) * nrm;
+  };
+  const double ek = fine_edge(rp.knn);
+  const double dk = radius_of_search2(upper(ek), metric);
+  const double bw = rp.decay >= 0 ? fmax(dk * rp.bw_scale, rp.bw_floor) : 0.0;
+  const double dkmax = (rp.decay >= 0 && rp.kmax <= (int64_t)rp.knn)
+                           ? radius_of_search2(upper(fine_edge(rp.kmax)), metric) : DBL_MAX * 2.0;
+  const double r = collect_radius(rp, dk, bw, false, dkmax);
+  const double E = metric == 2 ? p.eps_rel * ek / p.s2 + nrm * 0x1p-23 : p.eps_rel * nrm;
+  const float l2 = collect_limit(r, metric, E, p.eps_rel);
+  p.lim2[i] = l2;
+  // ball size: every point with w under the lower edge of the limit's bin is in the ball, every point of the ball has w
+  // under its upper edge.  Coarse counts are complete below the crossing + margin octaves (the sweep's top edge never
+  // fell below it); above, only the lower bound is known (ball_hi = -1).
+  const float ls = l2 * p.s2;
+  int64_t lo, hi = -1;
+  if (ls < 0.5f * t) {
+    lo = 0;
+    hi = hf[0];
+  } else if (ls < t) {
+    const int j = (int)((__float_as_uint(ls) >> 19) & 15u);          // sub-bin of the limit
+    lo = hf[0];
+    for (int b = 0; b < j; ++b) lo += hf[1 + b];
+    hi = lo + hf[1 + j];
+  } else {
+    const int e = (int)(__float_as_uint(ls) >> 23);
+    const int bl = min(max(e - p.elo, 0), 63);
+    const int bmax = bc + p.margin - 1;                  // last coarse bin counted in full
+    int64_t c = 0;
+    lo = 0;
+    for (int b = 0; b <= min(bl, bmax); ++b) {
+      if (b < bl) lo = c + hc[b];
+      c += hc[b];
+    }
+    if (bl <= bmax && bl < 63) hi = c;
+  }
+  p.ball_lo[i] = (int32_t)(lo < p.nr ? lo : p.nr);
+  p.ball_hi[i] = hi < 0 ? -1 : (int32_t)(hi < p.nr ? hi : p.nr);
+}
+
 RowParams make_row_params(const void* Xq, const void* Xr, int d, int knn, int64_t kmax, double decay,
                           double thresh, const double* bw_fixed, int bw_mode, double bw_scale, int metric) {
   RowParams rp;
@@ -763,5 +891,28 @@ extern "C" int gtb_csr_gather(const int32_t* st_idx, const double* st_val, const
                                                      out_idx, out_val);
     GTB_CHECK_LAUNCH();
   }
+  return GTB_OK;
+}
+
+extern "C" int gtb_knn_count_bound(const uint32_t* coarse, const uint32_t* fine, int64_t nq, int64_t nr, int elo,
+                                   int margin, float s2, const float* qn2, float maxrn2, double eps_rel, int x_kind,
+                                   int knn, int64_t kmax, double decay, double thresh, const double* bw_fixed,
+                                   int bw_mode, double bw_scale, float* top, float* lim2, int32_t* ball_lo,
+                                   int32_t* ball_hi, void* stream) {
+  GTB_CHECK_ARG(nq > 0 && nr > 0 && knn >= 1 && s2 > 0.f, "bad shape");
+  GTB_CHECK_ARG(x_kind >= 0 && x_kind <= 9, "x_kind: bit 0 = float64 rows, bits 1-3 = metric");
+  GTB_CHECK_ARG(coarse != nullptr || (bw_mode != 0 && decay >= 0 && lim2),
+                "without a coarse histogram: a fixed bandwidth (bw_mode 1 or 2) and lim2");
+  GTB_CHECK_ARG(coarse == nullptr || fine != nullptr || top, "coarse only: top is required");
+  GTB_CHECK_ARG(coarse == nullptr || fine == nullptr || (lim2 && ball_lo && ball_hi), "lim2, ball_lo, ball_hi required");
+  GTB_CHECK_ARG(elo >= 1 && elo + 64 <= 254 && margin >= 1, "1 <= elo <= 190, margin >= 1");
+  GTB_CHECK_ARG(decay < 0 || (thresh > 0 && thresh <= 1), "thresh must be in (0, 1]");
+  BoundParams p;
+  p.rp = make_row_params(nullptr, nullptr, 0, knn, kmax, decay, thresh, bw_fixed, bw_mode, bw_scale, x_kind >> 1);
+  p.coarse = coarse; p.fine = fine; p.nq = nq; p.nr = nr; p.elo = elo; p.margin = margin; p.s2 = s2;
+  p.qn2 = qn2; p.maxrn2 = maxrn2; p.eps_rel = eps_rel;
+  p.top = top; p.lim2 = lim2; p.ball_lo = ball_lo; p.ball_hi = ball_hi;
+  count_bound_kernel<<<(unsigned)gtb_cdiv(nq, 256), 256, 0, (cudaStream_t)stream>>>(p);
+  GTB_CHECK_LAUNCH();
   return GTB_OK;
 }

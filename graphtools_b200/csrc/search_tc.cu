@@ -34,6 +34,9 @@
 // per-lane predicated stores when many rows hit; a buffer that nears capacity is compacted to its LS smallest by
 // a warp-cooperative quickselect on 64-bit ordered keys (ballots and popcounts only) and the threshold tightens.
 // RADIUS mode: values under the row's limit are appended to the global pair list.
+// COUNT mode: values under the row's top edge are counted into a per-row histogram of their float32 bits in shared
+// memory (the rare-hit structure of TOPK: one min tree and ballot per batch, increments only for hits), added into a
+// caller-owned global histogram at the end of each round.
 //
 // Replaces sklearn ArgKmin / RadiusNeighbors behind knn_tree.kneighbors / radius_neighbors
 // (reference graphtools/graphs.py:883, :922, :957, :966).
@@ -90,6 +93,9 @@ struct TcParams {
   const float* qn2;
   int32_t* cand_idx; uint2* cand_buf; float* tau;          // TOPK: out [nq][2*TC_S], scratch [nq_pad][2][TC_CAP], tau [nq][2]
   const float* lim2; int2* pairs; unsigned long long capacity; unsigned long long* counter; int32_t* rowcnt;
+  // COUNT: hist [nq_pad][count_bins] (added to), top = per-row top edge of the fine pass (NULL: coarse pass), count_k =
+  // knn_eff, count_margin = octaves kept above the crossing, count_elo = exponent field of the coarse window's bin 1
+  uint32_t* hist; const float* top; int count_k, count_margin, count_elo, count_bins;
 };
 
 // ---------------------------------------------------------------- warp-cooperative compaction
@@ -242,7 +248,7 @@ __device__ __forceinline__ void tc_commit_mc_pred(uint32_t bar, uint16_t mask, u
 // lives in TMEM (hi parts only: 8 columns per k-step, up to 256 columns beside two accumulators), the reference tiles
 // stream in CHUNKS of 8 k-steps -- a stage is one (tile, chunk) pair and the accumulator collects all chunks of a tile.
 template <int MODE, int CL, int FMT, int LS, int QT, bool PIECE = false, bool WIDE = false,   // MODE 0 = TOPK, 1 = RADIUS,
-          bool LISTED = false>                                                                   // 2 = SEED
+          bool LISTED = false>                                                                   // 2 = SEED, 3 = COUNT
 __global__ void __launch_bounds__(TC_THREADS, 1)
 search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant__ CUtensorMap mBht,
                  const __grid_constant__ CUtensorMap mBl, const __grid_constant__ CUtensorMap mBlt,
@@ -262,6 +268,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
   static_assert(FMT != 3 || QT == 2, "the one-product flavour runs two query tiles per CTA");
   static_assert(!WIDE || (FMT == 2 && QT == 1 && !PIECE), "wide operand rows: fp16x2, one query tile per CTA");
   static_assert(!LISTED || (MODE == 0 && FMT == 3 && !PIECE && !WIDE), "tile lists: one-product top-k sweep");
+  static_assert(MODE != 3 || (FMT == 2 && QT == 1 && !PIECE && !LISTED), "count sweeps: fp16x2, one query tile per CTA");
   constexpr int LSO = (QT == 2) ? 2 * LS : LS;               // entries of one output list
   // candidate buffer of one list: a row owns TC_GROUPS * TC_CAP slots of scratch; the single long list of QT == 2 may
   // use all of them (fewer compactions between the seeded threshold and the final selection)
@@ -304,7 +311,7 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
   const int64_t nrounds = p.nrounds;
   const int64_t qcluster = cluster_id % p.n_qclusters;
   const int64_t tile0 = (cluster_id / p.n_qclusters) * p.tiles_per_split;
-  const int64_t tstride = (MODE != 1) ? p.tile_stride : 1;
+  const int64_t tstride = (MODE != 1 && MODE != 3) ? p.tile_stride : 1;
   const int64_t tiles_left = (p.nr_pad / TC_N + tstride - 1) / tstride - tile0;
   const int64_t ntiles = tiles_left < p.tiles_per_split ? tiles_left : p.tiles_per_split;
   // LISTED: the unit of a round (slots past the last unit are padding units: rows beyond nq_pad, no tiles) and its list
@@ -581,6 +588,11 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
     const int lgrp = (QT == 2) ? 0 : grp;            // list index inside a row's candidate storage
     const uint32_t a_col0 = (uint32_t)(my_qt * 64);
     int64_t it_run = 0;                              // LISTED: tiles of the earlier rounds (lists differ in length)
+    // COUNT: one [bins][128] histogram per CTA behind the transpose slots, shared by both groups (atomic increments)
+    uint32_t* hist_s = reinterpret_cast<uint32_t*>(gbase + (bar0 - base) + 256 + 1024);
+    if (MODE == 3) {
+      for (int i = threadIdx.x - 64; i < p.count_bins * TC_M; i += 128 * TC_GROUPS) hist_s[i] = 0u;
+    }
     for (int64_t round = 0; round < nrounds; ++round) {
     int64_t nt = ntiles, lo = 0;
     if (LISTED) { const int64_t u = unit_of(round); lo = list_lo(u); nt = list_len(u); }
@@ -605,9 +617,11 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_a);
     }
+    if (MODE == 3) asm volatile("bar.sync 1, 256;" ::: "memory");   // the previous round's histogram is flushed
 
     const float nx = valid ? p.qn2[gq] : 0.f;
     float thr;
+    int eo = 0;                                      // COUNT, fine pass: exponent field of the row's octave
     if (MODE == 0) {
       thr = valid ? BIG : -gtb_inf_f();
       if (valid && p.seed_tau != nullptr) {
@@ -619,6 +633,12 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
       // capped at BIG: every real value stays below it and every padded reference row above it, so a radius wider
       // than the data (a kernel support beyond all points) cannot admit padded columns j >= nr
       thr = valid ? fminf(p.lim2[gq] - nx, BIG) : -gtb_inf_f();
+    } else if (MODE == 3) {
+      // coarse pass: no top edge until the row's count reaches k; fine pass: the octave top t from the coarse pass
+      // (a row without one, t = +inf, is not counted: its limit is +inf whatever the fine pass finds)
+      const float t = (valid && p.top != nullptr) ? p.top[gq] : gtb_inf_f();
+      thr = (valid && (p.top == nullptr || t < gtb_inf_f())) ? fminf(t - nx, BIG) : -gtb_inf_f();
+      eo = (int)(__float_as_uint(t) >> 23) - 1;
     } else {
       thr = 0.f;
     }
@@ -676,6 +696,44 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
           const float lo = fminf(best[i], v);
           v = fmaxf(best[i], v);
           best[i] = lo;
+        }
+        continue;
+      }
+      if (MODE == 3) {
+        const float bm = fminf(fminf(tmin32(r0), tmin32(r1)), fminf(tmin32(r2), tmin32(r3)));
+        if (__ballot_sync(0xffffffffu, bm < thr) == 0u) continue;
+        // bins of w = v + |x|^2, the approximate squared distance (search units).  Coarse: bin = exponent field - elo,
+        // clamped to [0, 63] (zero and negative values: bin 0).  Fine: below the octave [t/2, t) -> 0, inside it
+        // 1 + the top four mantissa bits.
+        bool hit = false;
+#pragma unroll
+        for (int part = 0; part < TC_N / 32; ++part) {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const float v = __uint_as_float(part == 0 ? r0[j] : part == 1 ? r1[j] : part == 2 ? r2[j] : r3[j]);
+            if (v < thr) {
+              const uint32_t bits = __float_as_uint(v + nx);
+              const int e = (int)bits >> 23;
+              int bin;
+              if (p.top == nullptr) bin = min(max(e - p.count_elo, 0), 63);
+              else bin = (e < eo) ? 0 : (e == eo ? 1 + (int)((bits >> 19) & 15u) : -1);
+              if (bin >= 0) atomicAdd(hist_s + bin * TC_M + row, 1u);
+              hit = true;
+            }
+          }
+        }
+        if (p.top == nullptr && hit) {
+          // coarse top edge: count_margin octaves above the first bin whose cumulative count reaches k.  Counts only
+          // grow, so the edge only falls, and every value under the final crossing + margin has been counted.
+          uint32_t c = 0u;
+          int b = 0;
+          for (; b < 63; ++b) {
+            c += hist_s[b * TC_M + row];
+            if (c >= (uint32_t)p.count_k) break;
+          }
+          const int tb = b + p.count_margin;
+          if (b < 63 && tb < 63)
+            thr = fminf(thr, __uint_as_float((uint32_t)(p.count_elo + tb + 1) << 23) - nx);
         }
         continue;
       }
@@ -771,6 +829,20 @@ search_tc_kernel(const __grid_constant__ CUtensorMap mBh, const __grid_constant_
       }
     }
 
+    if (MODE == 3) {
+      // both groups are done with this round: add the CTA's counts into the global histogram and clear them
+      asm volatile("bar.sync 1, 256;" ::: "memory");
+      const int fr = (threadIdx.x - 64) & (TC_M - 1), half = (threadIdx.x - 64) >> 7;
+      const int64_t fq = q0 + fr;
+      const int nb = p.count_bins, b0 = half ? nb / 2 : 0, b1 = half ? nb : nb / 2;
+      for (int b = b0; b < b1; ++b) {
+        const uint32_t c = hist_s[b * TC_M + fr];
+        if (c) {
+          if (fq < p.nq) atomicAdd(p.hist + fq * nb + b, c);
+          hist_s[b * TC_M + fr] = 0u;
+        }
+      }
+    }
     if (MODE == 2) {
       if (valid) {
         const float tv = (best[TC_SEED_K - 1] >= BIG) ? gtb_inf_f() : best[TC_SEED_K - 1] + nx;
@@ -999,7 +1071,8 @@ int launch_tc_cl(const void* q_hi, const void* q_lo, const void* r_hi, const voi
   if ((rc = make_map(&mBlt, r_lo, p.nr_pad, Kp, EPK, TC_N / CL, false, FMT))) return rc;
   constexpr int NPART = (FMT == 3) ? 1 : 2;
   constexpr int NS = BF16 ? (NPART == 1 ? 4 : 3) : 2;
-  size_t smem = 1024 + (size_t)NPART * NS * TC_N * (WIDE ? 8 : p.nks) * 32 + 256 + 1024;
+  size_t smem = 1024 + (size_t)NPART * NS * TC_N * (WIDE ? 8 : p.nks) * 32 + 256 + 1024 +
+                (MODE == 3 ? (size_t)64 * TC_M * sizeof(uint32_t) : 0);
   auto kern = search_tc_kernel<MODE, CL, FMT, LS, QT, false, WIDE>;
   GTB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int dev = 0, nsm = 0;
@@ -1008,12 +1081,12 @@ int launch_tc_cl(const void* q_hi, const void* q_lo, const void* r_hi, const voi
   const int64_t n_cluster_tiles = gtb_cdiv(p.nq_pad / TC_M, CL * QT);
   int64_t n_clusters = n_cluster_tiles < (nsm / CL) ? n_cluster_tiles : (nsm / CL);
   p.nrounds = gtb_cdiv(n_cluster_tiles, n_clusters);
-  if (p.tile_stride < 1 || MODE == 1) p.tile_stride = 1;
+  if (p.tile_stride < 1 || MODE == 1 || MODE == 3) p.tile_stride = 1;
   const int64_t total_tiles = gtb_cdiv(p.nr_pad / TC_N, p.tile_stride);
   p.n_qclusters = n_clusters;
   p.tiles_per_split = total_tiles;
   int64_t splits = 1;
-  if (MODE == 1 && n_cluster_tiles * 2 <= nsm / CL && total_tiles >= 16) {
+  if ((MODE == 1 || MODE == 3) && n_cluster_tiles * 2 <= nsm / CL && total_tiles >= 16) {
     splits = (nsm / CL) / n_cluster_tiles;
     if (splits > total_tiles / 8) splits = total_tiles / 8;
     p.tiles_per_split = gtb_cdiv(total_tiles, splits);
@@ -1310,4 +1383,31 @@ extern "C" int gtb_knn_radius_tc(const void* q_hi, const void* q_lo, const float
   p.pairs = reinterpret_cast<int2*>(pairs); p.capacity = (unsigned long long)capacity; p.counter = counter;
   p.rowcnt = rowcnt; p.sync_ctr = pace; p.tile_stride = 1;
   return launch_tc<1>(q_hi, q_lo, r_hi, r_lo, Kp, dtype, 32, cluster, 1, p, (cudaStream_t)stream);
+}
+
+// Histogram count sweep (COUNT mode) on the fp16x2 operands of gtb_knn_radius_tc.  top == NULL: coarse pass, 64 bins
+// per row (float32 exponent fields elo - 1 + b of the approximate squared distance, bin 0 everything below, bin 63
+// everything above), counting stops count_margin octaves above the first bin whose cumulative count reaches k;
+// otherwise fine pass, 17 bins: below the octave [top/2, top), then its 16 sub-bins.  hist [nq_pad][bins] is zeroed
+// here and filled with atomics, so the counts do not depend on the tiling.
+extern "C" int gtb_knn_count_tc(const void* q_hi, const void* q_lo, const float* qn2, const float* top, int64_t nq,
+                                int64_t nq_pad, const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp,
+                                int dtype, int cluster, int k, int margin, int elo, uint32_t* hist, unsigned int* pace,
+                                void* stream) {
+  int rc = tc_check(nq, nr, nq_pad, nr_pad, Kp, dtype);
+  if (rc) return rc;
+  GTB_CHECK_ARG(dtype == 2, "count sweeps run on the fp16x2 operands (dtype 2)");
+  GTB_CHECK_ARG(cluster == 1 || cluster == 2, "cluster size must be 1 or 2");
+  GTB_CHECK_ARG(k >= 1 && margin >= 1 && elo >= 1 && elo + 64 <= 254, "k >= 1, margin >= 1, 1 <= elo <= 190");
+  TcParams p{};
+  p.nq = nq; p.nq_pad = nq_pad; p.nr = nr; p.nr_pad = nr_pad; p.qn2 = qn2; p.sync_ctr = pace; p.tile_stride = 1;
+  p.hist = hist; p.top = top; p.count_k = k; p.count_margin = margin; p.count_elo = elo;
+  p.count_bins = top ? 17 : 64;
+  cudaStream_t st = (cudaStream_t)stream;
+  GTB_CUDA(cudaMemsetAsync(hist, 0, sizeof(uint32_t) * nq_pad * p.count_bins, st));
+  if (Kp > 128)
+    return cluster == 1 ? launch_tc_cl<3, 1, 2, 32, 1, true>(q_hi, q_lo, r_hi, r_lo, Kp, p, st)
+                        : launch_tc_cl<3, 2, 2, 32, 1, true>(q_hi, q_lo, r_hi, r_lo, Kp, p, st);
+  return cluster == 1 ? launch_tc_cl<3, 1, 2, 32, 1>(q_hi, q_lo, r_hi, r_lo, Kp, p, st)
+                      : launch_tc_cl<3, 2, 2, 32, 1>(q_hi, q_lo, r_hi, r_lo, Kp, p, st);
 }

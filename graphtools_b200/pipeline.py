@@ -429,6 +429,42 @@ def choose_S(knn_eff, binary):
         "knn={} needs a candidate list longer than 128; not supported by the fused top-k yet".format(knn_eff))
 
 
+def wide_knn(knn, binary):
+    """Whether a kNN search needs more neighbours than the candidate lists hold (exactly where choose_S raises): such
+    rows are bounded by histogram count sweeps and finished by the radius pass (knn_kernel)."""
+    return knn + (4 if binary else 8) > 128
+
+
+def count_flavour(want, d, metric):
+    """Flavour of the count and collect sweeps of a wide-knn build: fp16x2 ("tch") where the radius pass of
+    GTB_SEARCH_IMPL=``want`` would run on the float16 operands (its first flavour that fits ``d`` is tch1 or tch), the
+    CUDA cores ("simt") otherwise -- cityblock, feature counts no tensor-core flavour takes, and the tc / tc16
+    preferences (the count mode exists for the fp16x2 operands only; one flavour for all three sweeps keeps one
+    rounding bound)."""
+    if metric == "cityblock":
+        return "simt"
+    if want not in FALLBACK:
+        raise ValueError("GTB_SEARCH_IMPL must be auto, tc, tc16, tch, tch1 or simt (got %r)" % (want,))
+    impl = next(c for c in FALLBACK[want] if c == "simt" or FLAVOURS[c].fits(d))
+    return "tch" if impl in ("tch1", "tch") else "simt"
+
+
+def count_window(vmax):
+    """Exponent field of bin 1 of the coarse histogram (elo): ``vmax``, an upper bound on every approximate squared
+    distance of the sweep in search units, lands in bin 62 at the latest, so bin 63 stays empty of real values."""
+    if not (vmax > 0):
+        return 1
+    m, e = math.frexp(vmax)                      # vmax = m 2^e, 0.5 <= m < 1: exponent field e - 1 + 127
+    return int(min(max(e + 126 - 62, 1), 190))
+
+
+def count_margin(f):
+    """Octaves the coarse count keeps above its crossing: the collect limit is at most ``f`` (>= 1, search units) times
+    the knn-th bound, and its bin must lie in the fully counted range (one octave for the bound's own bin, one more for
+    the rounding bound E)."""
+    return int(min(2 + max(0, math.ceil(math.log2(f))), 62))
+
+
 def default_impl():
     """GTB_SEARCH_IMPL = tc (3xTF32 tensor cores) | tc16 (bf16x3 tensor cores) | tch (fp16x2 tensor cores: two
     products, wider certified bound) | tch1 (fp16, ONE product, seeded thresholds, lists of 64) | simt (fp32 CUDA
@@ -685,9 +721,10 @@ def _sweep_simt(plan, qry, ref):
     return cand, tau, qry.n2, eps_rel_simt(ref.d), 1.0
 
 
-def _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out, nzero, x64, kern):
+def _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out, nzero, x64, kern, capacity=None):
     """Rows the refine could not certify: every reference point inside the row's radius ``lim2``, refined in float64
-    and merged into ``n_keep`` / ``bw_out`` / ``nzero``.  Returns the rows' segments (ptr, idx, val, n_keep)."""
+    and merged into ``n_keep`` / ``bw_out`` / ``nzero``.  Returns the rows' segments (ptr, idx, val, n_keep).
+    ``capacity``: pairs to allocate for the first attempt (default from the list length)."""
     nr, d = ref.n, ref.d
     nt = todo_rows.shape[0]
     nt_pad = (nt + 127) // 128 * 128
@@ -707,7 +744,7 @@ def _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out,
         QT = _empty((ref.d_pad, nt_pad), torch.float32)
         qn2 = _empty((nt_pad,), torch.float32)
         E.call("gtb_gather_operand", qry.XT, qry.n_pad, qry.n2, todo_rows, nt, QT, nt_pad, ref.d_pad, qn2)
-    capacity = max(1 << 20, nt * 4 * plan.S)
+    capacity = max(1 << 20, nt * 4 * plan.S) if capacity is None else max(1, capacity)
     while True:
         pairs = _empty((capacity, 2), torch.int32)
         counter = _zeros((1,), torch.int64)
@@ -735,6 +772,7 @@ def _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out,
     n_keep_t = _empty((nt,), torch.int32)
     overflow = _empty((1,), torch.int32)
     longest = int(rowcnt.max().item())
+    _STATS.update(ball_max=longest, ball_mean=npairs / nt)
     cap = 64
     while cap < longest:
         cap *= 2
@@ -766,9 +804,6 @@ def knn_kernel(ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandw
     kmax = 0 if knn_max is None else int(knn_max)
     if kmax >= nr:
         kmax = 0
-    plan = plan_search(default_impl(), d, ref.n_pad, ref.metric, knn, kmax, binary)
-    sweep = _sweep_simt if plan.impl == "simt" else _sweep_tc
-    cand, tau, q_n2, eps_rel, scale = sweep(plan, qry, ref)
 
     # bandwidth argument
     bw_mode, bw_fixed = 0, None
@@ -784,6 +819,12 @@ def knn_kernel(ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandw
     # kernel parameters, in the order both refine entry points take them
     kern = (knn, kmax, -1.0 if binary else float(decay), 1.0 if binary else float(thresh), bw_fixed, bw_mode,
             float(bandwidth_scale))
+    if wide_knn(knn, binary):
+        return _knn_kernel_wide(ref, qry, kern, x64)
+
+    plan = plan_search(default_impl(), d, ref.n_pad, ref.metric, knn, kmax, binary)
+    sweep = _sweep_simt if plan.impl == "simt" else _sweep_tc
+    cand, tau, q_n2, eps_rel, scale = sweep(plan, qry, ref)
 
     S = plan.S
     st_idx = _empty((nq, S), torch.int32)
@@ -801,7 +842,8 @@ def knn_kernel(ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandw
     count = _empty((1,), torch.int32)
     E.call("gtb_compact_todo", status, nq, todo_rows, count)
     nt = int(count.item())                       # host sync #1
-    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=plan.impl, euclidean_fallback_rows=0)
+    _STATS.update(rows=nq, radius_rows=nt, S=S, radius_pairs=0, impl=plan.impl, euclidean_fallback_rows=0,
+                  wide_knn=False, count_sweeps=0, ball_max=None, ball_mean=None)
 
     seg = (None,) * 4
     if nt > 0:
@@ -817,6 +859,97 @@ def knn_kernel(ref, qry=None, *, knn, knn_max=None, decay=40, thresh=1e-4, bandw
     _STATS.update(nnz_raw=nnz)
     csr = DeviceCSR(indptr, out_idx, out_val, (nq, nr))
     return csr, {"bandwidth": bw_out, "nzero": nzero}
+
+
+def _knn_kernel_wide(ref, qry, kern, x64):
+    """knn_kernel for knn beyond the candidate lists (wide_knn): no list and no stage-1 refine.  Every row goes through
+    the radius pass.  Its limit comes from the kernel support alone under a fixed bandwidth; with the adaptive bandwidth
+    (and for binary kNN) the knn-th distance is first bounded by two histogram count sweeps -- coarse (one bin per octave
+    of the approximate squared distance) and fine (16 sub-bins of the octave where the row's count reaches knn) -- and
+    gtb_knn_count_bound turns the bound into the limit by the refine's own status-2 rule (csrc/refine.cu)."""
+    knn, kmax, decay, thresh, bw_fixed, bw_mode, bw_scale = kern
+    binary = decay < 0
+    nq, nr, d = qry.n, ref.n, ref.d
+    flav = count_flavour(default_impl(), d, ref.metric)
+    f = FLAVOURS.get(flav)
+    plan = SearchPlan(flav, None, None, knn, 1, False)
+    _STATS.update(rows=nq, radius_rows=nq, S=None, radius_pairs=0, impl=flav, euclidean_fallback_rows=0, wide_knn=True,
+                  count_sweeps=0, ball_max=None, ball_mean=None)
+    scale = fp16_scale(max(qry.norm_max(), ref.norm_max())) if f else 1.0
+    s2 = scale * scale
+    l1 = ref.metric == "cityblock"
+    # the rounding bound of the sweeps: the arguments gtb_refine_topk takes after the same sweep
+    if l1:
+        q_n2 = qry.l1_norms()[0] if ref.is64 else None
+        maxnorm, eps_rel = (ref.l1_norms()[1] if ref.is64 else 0.0), eps_rel_l1(d)
+    elif f:
+        q_hi, q_lo, q_n2 = qry.tc(0, f.dtype, scale)
+        r_hi, r_lo, _ = ref.tc(1, f.dtype, scale)
+        maxnorm, eps_rel = ref.maxnorm, f.eps_rel(d)
+    else:
+        q_n2, maxnorm, eps_rel = qry.n2, ref.maxnorm, eps_rel_simt(d)
+    lim2 = _empty((nq,), torch.float32)
+    capacity = None
+    if bw_mode != 0:
+        E.call("gtb_knn_count_bound", None, None, nq, nr, 1, 1, 1.0, q_n2, maxnorm, eps_rel, x64, knn, kmax, decay, thresh,
+               bw_fixed, bw_mode, bw_scale, None, lim2, None, None)
+        capacity = max(1 << 20, nq * knn)
+    else:
+        if l1:
+            vmax = 1.01 * (qry.l1_norms()[1] + ref.l1_norms()[1])
+        else:
+            vmax = 4.04 * max(qry.maxnorm, ref.maxnorm) * s2
+        elo = count_window(vmax)
+        rf = 1.0 if binary else max(1.0, bw_scale * (-math.log(thresh)) ** (1.0 / decay))
+        margin = count_margin(rf * rf if ref.metric == "euclidean" else rf)
+        hists = []
+        top = None
+        for bins in (64, 17):                         # coarse, then fine from the coarse crossings
+            h = _empty((qry.n_pad, bins), torch.int32)
+            tag = "#coarse" if top is None else "#fine"
+            if f:
+                pace = _empty((1,), torch.int32)
+                E.call("gtb_knn_count_tc" + tag, q_hi, q_lo, q_n2 * s2, top, nq, qry.n_pad, r_hi, r_lo, nr, ref.n_pad,
+                       ref.kp(f.dtype), f.dtype, TC_CLUSTER, knn, margin, elo, h, pace)
+            elif l1:
+                E.call("gtb_knn_count_simt" + tag, qry.XT, None, top, nq, qry.n_pad, ref.XT, None, nr, ref.n_pad, ref.d_pad,
+                       knn, margin, elo, h)
+            else:
+                E.call("gtb_knn_count_simt" + tag, qry.XT, qry.n2, top, nq, qry.n_pad, ref.XT, ref.n2, nr, ref.n_pad,
+                       ref.d_pad, knn, margin, elo, h)
+            hists.append(h)
+            if top is None:
+                top = _empty((nq,), torch.float32)
+                E.call("gtb_knn_count_bound", h, None, nq, nr, elo, margin, s2, q_n2, maxnorm, eps_rel, x64, knn, kmax,
+                       decay, thresh, None, 0, bw_scale, top, None, None, None)
+        _STATS.update(count_sweeps=2)
+        ball_lo = _empty((nq,), torch.int32)
+        ball_hi = _empty((nq,), torch.int32)
+        E.call("gtb_knn_count_bound", hists[0], hists[1], nq, nr, elo, margin, s2, q_n2, maxnorm, eps_rel, x64, knn,
+               kmax, decay, thresh, None, 0, bw_scale, None, lim2, ball_lo, ball_hi)
+        lo_max, hi_min, hi_sum = (int(v) for v in torch.stack(
+            [ball_lo.max().long(), ball_hi.min().long(), ball_hi.long().sum()]).cpu())
+        if lo_max > BALL_CAP:
+            # the ball of this row is known to be too long before any pair is collected
+            raise RowTooLong(
+                "a row has {} neighbours inside the kernel radius; the sparse kNN pipeline handles rows of up to {} "
+                "(a kernel this dense calls for graphtype='exact', which evaluates every pair)".format(lo_max, BALL_CAP))
+        if hi_min >= 0:
+            capacity = hi_sum                         # every row's ball size is bounded: the pair list fits exactly
+    status = torch.full((nq,), 2 if bw_mode == 0 else 0, dtype=torch.int32, device=_dev())
+    todo_rows = torch.arange(nq, dtype=torch.int32, device=_dev())
+    n_keep = _empty((nq,), torch.int32)
+    bw_out = _empty((nq,), torch.float64)
+    nzero = _empty((nq,), torch.int32)
+    seg = _radius_pass(plan, qry, ref, scale, todo_rows, lim2, status, n_keep, bw_out, nzero, x64, kern,
+                       capacity=capacity)
+    indptr = exclusive_scan(n_keep)
+    nnz = int(indptr[-1].item())
+    out_idx = _empty((nnz,), torch.int32)
+    out_val = _empty((nnz,), torch.float64)
+    E.call("gtb_csr_gather", None, None, n_keep, status, indptr, nq, 0, todo_rows, nq, *seg, out_idx, out_val)
+    _STATS.update(nnz_raw=nnz)
+    return DeviceCSR(indptr, out_idx, out_val, (nq, nr)), {"bandwidth": bw_out, "nzero": nzero}
 
 
 def sort_rows(ptr, idx, val, n):

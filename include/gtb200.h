@@ -144,6 +144,19 @@ int gtb_knn_radius_tc(const void* q_hi, const void* q_lo, const float* qn2, cons
                       int64_t nq_pad, const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp,
                       int dtype, int cluster, int32_t* pairs, int64_t capacity, unsigned long long* counter,
                       int32_t* rowcnt, unsigned int* pace, void* stream);
+/* Histogram count sweeps (kNN graphs whose knn is beyond the candidate lists): per query row, counts of the approximate
+ * squared distances w (search units) by float32 bits, into hist[nq_pad][bins] (zeroed by the call, filled with
+ * atomics).  top == NULL: coarse pass, 64 bins: bin b holds exponent field elo + b (bin 0 everything below, bin 63
+ * everything above); counting stops `margin` octaves above the first bin whose cumulative count reaches k.  Otherwise
+ * fine pass, 17 bins: w < top[i]/2, then the 16 sub-bins of [top[i]/2, top[i]) by the top four mantissa bits (rows
+ * with top = +inf are not counted).  _tc: the fp16x2 operands of gtb_knn_radius_tc (dtype 2); _simt: the operands of
+ * gtb_knn_radius_simt, or with qn2 = rn2 = NULL those of gtb_knn_radius_simt_l1 (cityblock distances). */
+int gtb_knn_count_tc(const void* q_hi, const void* q_lo, const float* qn2, const float* top, int64_t nq, int64_t nq_pad,
+                     const void* r_hi, const void* r_lo, int64_t nr, int64_t nr_pad, int Kp, int dtype, int cluster,
+                     int k, int margin, int elo, uint32_t* hist, unsigned int* pace, void* stream);
+int gtb_knn_count_simt(const float* QT, const float* qn2, const float* top, int64_t nq, int64_t nq_pad,
+                       const float* RT, const float* rn2, int64_t nr, int64_t nr_pad, int d_pad, int k, int margin,
+                       int elo, uint32_t* hist, void* stream);
 
 /* ---- K3 float64 re-evaluation, bandwidth, affinities, CSR emission: replaces graphs.py:886-911
  * and _build_csr_from_neighbors (graphs.py:450-559) ------------------------------------------ */
@@ -177,6 +190,16 @@ int gtb_csr_gather(const int32_t* st_idx, const double* st_val, const int32_t* n
                    const int64_t* indptr, int64_t nq, int S, const int32_t* todo_rows, int64_t nt,
                    const int64_t* seg_ptr, const int32_t* seg_idx, const double* seg_val,
                    const int32_t* n_keep_t, int32_t* out_idx, double* out_val, void* stream);
+/* Collect limits of the count path (rows whose knn is beyond the candidate lists), by the rule of the status-2 rows of
+ * gtb_refine_topk with the knn-th distance bounded from the histograms: fine == NULL: top[nq] = upper edge of the
+ * first coarse bin whose cumulative count reaches knn (+inf: none); otherwise lim2[nq] (data units, as lim2_out) and
+ * bounds on the ball size: ball_lo <= |ball| <= ball_hi (-1: not known).  s2: search units per data unit (fp16 scale
+ * squared, else 1); qn2 / maxrn2 / eps_rel / x_kind as for gtb_refine_topk.  coarse == NULL: fixed bandwidth
+ * (bw_mode 1 or 2), lim2 = the kernel support alone. */
+int gtb_knn_count_bound(const uint32_t* coarse, const uint32_t* fine, int64_t nq, int64_t nr, int elo, int margin,
+                        float s2, const float* qn2, float maxrn2, double eps_rel, int x_kind, int knn, int64_t kmax,
+                        double decay, double thresh, const double* bw_fixed, int bw_mode, double bw_scale, float* top,
+                        float* lim2, int32_t* ball_lo, int32_t* ball_hi, void* stream);
 
 /* ---- K4 sparse symmetrise / normalise: replaces base.py:557-577, :579-592, :645, :648-666 --- */
 int64_t gtb_scan_ws_elems(int64_t n);
