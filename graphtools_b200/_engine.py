@@ -89,6 +89,10 @@ _SIGS = {
     "gtb_spmm_csr": ([_P, _P, _P, c_int64, _P, c_int64, c_int, _P, c_int64, _P], 1),
     "gtb_spmm_cheb": ([_P, _P, _P, c_int64, _P, c_int64, c_int, c_double, c_double, c_double, _P, c_int64, _P, c_int64,
                        _P], 1),
+    "gtb_spmm_cheb_acc": ([_P, _P, _P, c_int64, _P, c_int64, c_int, c_double, c_double, c_double, _P, c_int64, _P,
+                           c_int64, _P, c_int, _P, c_int64, c_int64, _P], 1),
+    "gtb_laplacian_count": ([_P, _P, _P, c_int64, _P, _P, _P], 1),
+    "gtb_laplacian_fill": ([_P, _P, _P, c_int64, _P, _P, c_int, _P, _P, _P], 1),
     "gtb_row_scale": ([_P, _P, c_int64, c_int, c_int, _P, _P], 1),
     "gtb_slice_f64": ([_P, c_int64, c_int64, c_int64, c_int, c_int, c_int64, c_int64, _P, _P, _P], 2),
     "gtb_gemm_i8": ([_P, _P, c_int, c_int64, c_int64, c_int64, c_int64, c_int64, _P, _P, _P, c_int64, c_int, _P], 1),

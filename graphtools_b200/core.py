@@ -614,6 +614,47 @@ class BaseGraph(Base, metaclass=abc.ABCMeta):
         return eigen.diffusion_map(self, n_components=n_components, t=t, tol=tol, maxiter=maxiter,
                                    random_state=random_state)
 
+    def laplacian(self, lap_type="combinatorial"):
+        """Graph Laplacian of W = K without its diagonal (pygsp's ``compute_laplacian``): scipy CSR, float64, with
+        sorted int32 indices.  "combinatorial" is D - W, "normalized" is I - D^-1/2 W D^-1/2, where D holds the row
+        sums dw of W (added in column order); a vertex with dw = 0 gets L_ii = 0.  L stores K's off-diagonal pattern
+        and one diagonal entry per row.  Dense kernels and landmark graphs use their full kernel K.  Raises
+        ValueError for kernel_symm=None or an unknown ``lap_type``.  Built on the device (csrc/gsp.cu) and cached
+        there; on a row-sharded build the first call gathers the kernel (collective)."""
+        from . import gsp
+        return gsp.laplacian(self, lap_type)
+
+    def estimate_lmax(self, lap_type="combinatorial"):
+        """Upper estimate of the largest eigenvalue of ``laplacian(lap_type)``: 1.01 times the top Ritz value of
+        Lanczos on the device, capped at the bound 2 (normalized) or 2 max(dw) (combinatorial), as pygsp's
+        ``estimate_lmax``.  Reproducible from call to call, and cached per ``lap_type`` (gsp.py has the rules)."""
+        from . import gsp
+        gsp.check_lap_type(lap_type)
+        cache = self.__dict__.setdefault("_lmax", {})
+        if lap_type not in cache:
+            cache[lap_type] = float(gsp.estimate_lmax(self, lap_type))
+        return cache[lap_type]
+
+    def filter(self, signal, kernel, order=30, lap_type="combinatorial", lmax=None, return_device=False):
+        """Spectral filter h(L) applied to ``signal`` ([N] or [N, f], numpy or torch) by pygsp's Chebyshev
+        approximation of degree ``order`` on [0, lmax] (``compute_cheby_coeff`` and ``cheby_op``, same operation
+        order: bit-identical to that code on the host with the same lmax, signed zeros aside).  ``kernel`` is a
+        vectorised callable h(lambda) or a list of F of them; a list adds a trailing axis of size F to the result.
+        ``lmax=None`` uses ``estimate_lmax(lap_type)``.  Raises ValueError for kernel_symm=None, an unknown
+        ``lap_type``, order < 1, a signal of the wrong shape or with non-finite values, a kernel that is not callable
+        or returns non-finite or wrongly shaped values, and lmax <= 0.  Each recurrence step is one launch of the
+        fused filter step (csrc/spmm.cu, gsp.py)."""
+        from . import gsp
+        return gsp.filter(self, signal, kernel, order=order, lap_type=lap_type, lmax=lmax,
+                          return_device=return_device)
+
+    def heat_filter(self, signal, tau=10, order=30, lap_type="combinatorial", lmax=None, return_device=False):
+        """``filter`` with pygsp's heat kernel h(lambda) = exp(-tau lambda / lmax); a sequence of ``tau`` gives a
+        filter bank.  ``G.heat_filter(onehot_labels, tau=60, order=50)`` is the MELD-style use."""
+        from . import gsp
+        return gsp.heat_filter(self, signal, tau=tau, order=order, lap_type=lap_type, lmax=lmax,
+                               return_device=return_device)
+
     @staticmethod
     def _materialize(dev):
         if isinstance(dev, pipeline.DeviceCSR):

@@ -13,4 +13,4 @@ void gtb_set_error(const char* fmt, ...) {
 }
 
 extern "C" const char* gtb_last_error(void) { return g_err; }
-extern "C" int gtb_version(void) { return 205; }   // + gtb_knn_count_tc / _simt / _bound (knn beyond the lists)
+extern "C" int gtb_version(void) { return 206; }   // + gtb_spmm_cheb_acc, gtb_laplacian_count/_fill (csrc/gsp.cu)

@@ -324,6 +324,23 @@ int gtb_spmm_csr(const int64_t* indptr, const int32_t* idx, const double* val, i
 int gtb_spmm_cheb(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const double* Y,
                   int64_t ldy, int f, double alpha, double beta, double gamma, const double* Z, int64_t ldz,
                   double* out, int64_t ldo, void* stream);
+/* Step of a Chebyshev filter bank (graphtools_b200/gsp.py, pygsp's cheby_op): gtb_spmm_cheb's out, then for every
+ * a < F: R[a * ldrb + i * ldr + k] = R[...] + coef[a] * out[i][k] (product and sum rounded separately, numpy's
+ * `r += c * out`).  coef: F doubles in device memory; R: F blocks of [n][ldr] (first f columns), ldrb apart.  The
+ * aliasing rules of gtb_spmm_cheb hold; R overlapping Y, Z or out, blocks of R overlapping each other, and coef
+ * overlapping R or out are rejected (GTB_ERR_ARG). */
+int gtb_spmm_cheb_acc(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const double* Y,
+                      int64_t ldy, int f, double alpha, double beta, double gamma, const double* Z, int64_t ldz,
+                      double* out, int64_t ldo, const double* coef, int F, double* R, int64_t ldr, int64_t ldrb,
+                      void* stream);
+/* Graph Laplacian of a square column-sorted CSR kernel K, W = K without its diagonal (pygsp's compute_laplacian;
+ * csrc/gsp.cu): count writes dw[n] (sequential column-order sums of W's rows) and len[n] (row lengths of L: W's
+ * entries plus one diagonal); after gtb_exclusive_scan(len) -> lptr, fill writes L's column-sorted indices and
+ * values, lap_type 0 combinatorial (L = D - W) or 1 normalized (I - D^-1/2 W D^-1/2; zero-degree rows get L_ii = 0) */
+int gtb_laplacian_count(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, double* dw,
+                        int32_t* len, void* stream);
+int gtb_laplacian_fill(const int64_t* indptr, const int32_t* idx, const double* val, int64_t n, const double* dw,
+                       const int64_t* lptr, int lap_type, int32_t* lidx, double* lval, void* stream);
 /* out[i][:] = in[i][:] * s[i]   (power_neg_half = 0)   or   in[i][:] / sqrt(s[i])   (power_neg_half = 1) */
 int gtb_row_scale(const double* in, const double* s, int64_t n, int f, int power_neg_half, double* out,
                   void* stream);
